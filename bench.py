@@ -6,7 +6,7 @@ Workload at every N: BASELINE config 2 per GPU — wind_mixing u/v/T NDE forward
 columns x 1,152 steps, every frame saved (1.81 GB of trajectory per solve, larger than L2) — weak scaling: columns
 shard across ranks with no data-path collective. One bench "step" = one full solve of the rank's column batch.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Prints ONE JSON line (rank 0). `value` = device-resident throughput, `e2e` = through the host-pointer C ABI call
@@ -34,6 +34,7 @@ import numpy as np  # noqa: E402
 
 NCOL = 4096
 NSTEPS = 1152
+DUMP_COLUMNS = 64
 FP32_LANES_PER_SM = 128
 # ncu --set full summaries of the dominant kernel at the bench configuration (newest round first); `traffic` and the
 # tensor-pipe activity are READ from the committed file, not typed into this source
@@ -180,6 +181,16 @@ def build_workload(syn, RHS_INFER, n_steps):
     return d, theta
 
 
+def dump_outputs(out_dir, traj_d):
+    """The trajectory [columns, frames, S] of the last timed solve, as float32 .npy: the final frame of every column and
+    every frame of a fixed, seeded sample of DUMP_COLUMNS columns (about 30 MB; the whole trajectory is 1.81 GB)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cols = np.sort(np.random.default_rng(0).choice(traj_d.shape[0], DUMP_COLUMNS, replace=False))
+    np.save(os.path.join(out_dir, "final_state.npy"), traj_d[:, -1].cpu().numpy())
+    np.save(os.path.join(out_dir, "trajectory_sample.npy"), traj_d[torch.from_numpy(cols).to(traj_d.device)].cpu().numpy())
+
+
 def flops_per_colstep(d):
     mlp = 2 * sum(n.macs for n in d.nets)
     return (mlp + 1200) * d.rhs_evals_per_step
@@ -293,7 +304,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip adjoint / nn_free / cpu_baseline side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (rank 0's "
+                    "columns) to DIR/*.npy, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -362,6 +377,8 @@ def main():
     ms_total = float(t.item())
     colsteps_per_step = NCOL * NSTEPS * world
     value = colsteps_per_step * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, traj_d)
 
     # ---- end-to-end through the host-pointer C ABI (pinned host buffers; H2D + D2H inside the timed region) ----
     x0_h = torch.tensor(x0).pin_memory(); bcs_h = torch.tensor(bcs).pin_memory()

@@ -44,13 +44,19 @@ def config3_slice():
     return grad_case(d, th, x0, bcs, tgt, W3)
 
 
+def bench_targets(d, x0):
+    """bench.py's config-3 targets: a smooth drift of the initial profiles (cheap to rebuild, so not stored)."""
+    tgt = np.ascontiguousarray(np.repeat(x0[:, None, :], d.n_saved, axis=1))
+    return (tgt + 0.05 * np.linspace(0, 1, d.n_saved, dtype=np.float32)[None, :, None]).astype(np.float32)
+
+
 def config3_bench_theta():
     d = syn.wind_mixing_desc(variant=RHS_TRAIN, net="uvT_small", n_steps=1152, save_stride=9, ckpt_stride=1)
     th = syn.theta_init(d, seed=42, scale=1e-5)
     x0, bcs = syn.columns(d, 32, seed=1000)
-    tgt = np.ascontiguousarray(np.repeat(x0[:, None, :], d.n_saved, axis=1))
-    tgt = (tgt + 0.05 * np.linspace(0, 1, d.n_saved, dtype=np.float32)[None, :, None]).astype(np.float32)
-    return grad_case(d, th, x0, bcs, tgt, W3)
+    out = grad_case(d, th, x0, bcs, bench_targets(d, x0), W3)
+    del out["targets"]
+    return out
 
 
 def forward_case(d, th, ncol, seed=1000, frames=None):
@@ -102,7 +108,32 @@ CASES = {"fullsize_config1_random": lambda: config1(0.1), "fullsize_config1_init
          "fullsize_config2_undivided": config2_undivided, "fullsize_nnfree": nnfree_full,
          "fullsize_config4_init": lambda: config4_slice(1e-5), "fullsize_config4_random": lambda: config4_slice(0.1)}
 
+# arrays that do not compress below 1 MB: written in this many parts along the column axis, the first part in <name>.npz
+# with the other arrays, part i in <name>.<i>.npz
+SPLIT = {"fullsize_config3_slice": ("targets", 2), "fullsize_config4_random": ("traj", 2)}
+
+
+def save(name, out):
+    if name not in SPLIT:
+        np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
+        return
+    key, n = SPLIT[name]
+    parts = np.array_split(out[key], n)
+    np.savez_compressed(os.path.join(HERE, name + ".npz"), **{**out, key: parts[0]})
+    for i, part in enumerate(parts[1:], 1):
+        np.savez_compressed(os.path.join(HERE, f"{name}.{i}.npz"), **{key: part})
+
+
+def load(name):
+    """The arrays save() wrote for `name`, split arrays joined again."""
+    out = dict(np.load(os.path.join(HERE, name + ".npz")))
+    if name in SPLIT:
+        key, n = SPLIT[name]
+        out[key] = np.concatenate([out[key]] + [np.load(os.path.join(HERE, f"{name}.{i}.npz"))[key] for i in range(1, n)])
+    return out
+
+
 if __name__ == "__main__":
     for name in (sys.argv[1:] or CASES):
-        np.savez_compressed(os.path.join(HERE, name + ".npz"), **CASES[name]())
+        save(name, CASES[name]())
         print("wrote", name, flush=True)

@@ -8,17 +8,20 @@ horizon amplifies rounding through the tanh step of the Richardson-number diffus
 LONG_FLOOR_FACTOR x that floor: two FP32 evaluation orders of a sensitive map differ from the FP64 answer by amounts of
 the same size, not by identical amounts. This is a stated relaxation of the north-star number, reported in DESIGN.md."""
 import os
+import sys
 
 import numpy as np
 import pytest
 import torch
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+sys.path.insert(0, GOLDEN)
+import make_fullsize  # noqa: E402
 
 
 def golden(name):
     """FP64-oracle answers computed once by tests/golden/make_fullsize.py (minutes of CPU per case) and committed."""
-    return np.load(os.path.join(GOLDEN, name + ".npz"))
+    return make_fullsize.load(name)
 
 from cpz_b200 import engine, synthetic as syn
 from cpz_b200.desc import ClosureDesc, RHS_INFER, RHS_TRAIN
@@ -56,7 +59,7 @@ class _env:
 def config3_slice():
     """36 columns (one full 32-column tile + a ragged one) of BASELINE config 3 with un-divided weights (scale 0.1) so
     that the MLP contributes; targets = FP64 oracle solution of a perturbed theta (SURVEY 8d); FP64 loss / gradient and
-    the FP32-oracle floors from tests/golden/fullsize_config3_slice.npz."""
+    the FP32-oracle floors from tests/golden/fullsize_config3_slice*.npz."""
     d = syn.wind_mixing_desc(variant=RHS_TRAIN, net="uvT_small", n_steps=1152, save_stride=9, ckpt_stride=9)
     th = syn.theta_random(d, scale=0.1)
     x0, bcs = syn.columns(d, 36)
@@ -90,7 +93,7 @@ def test_grad_config3_bench_theta_full_length(ctx):
     th = syn.theta_init(d, seed=42, scale=1e-5)
     x0, bcs = syn.columns(d, 32, seed=1000)
     G = golden("fullsize_config3_bench_theta")
-    tgt, tot, g, floor = G["targets"], float(G["loss"][6]), G["grad"], float(G["floor_grad"])
+    tgt, tot, g, floor = make_fullsize.bench_targets(d, x0), float(G["loss"][6]), G["grad"], float(G["floor_grad"])
     for ckpt in (1, 9):
         d.ckpt_stride = ckpt
         m = engine.Model(ctx, d, th)
