@@ -641,6 +641,11 @@ constexpr int WG_NT = 576;    // two halves of 8 converter warps + one MMA-issui
 constexpr int WG_HT = 256;    // converter threads of a half
 constexpr int WG_BAR = 288;   // threads at a half's barrier
 constexpr int WG_COLS = 448;  // N1 + 2 N2 + 96 <= 448
+// Sub-records summed in tensor memory before the sums are added to the CTA's FP32 image. One accumulation over every record
+// of a launch loses accuracy with its length: at 2 304 columns x 124 steps (~1 500 sub-records per CTA) the weight gradient
+// was 1.5e-4 from FP64 where the FP32 oracle is 9e-6 off; blocks of 128 give 1.6e-5 (blocks of 32: 8e-6 at about twice the
+// cost). Measured on a B200 at 1000 W: the bench.py config-3 step takes 356 ms instead of 347 ms.
+constexpr int WG_BLOCK = 128;
 
 __device__ __forceinline__ uint64_t wg_desc(uint32_t saddr, uint32_t lbo_bytes) {  // K-major, no swizzle, SBO = 128
   return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16) | ((uint64_t)(128 >> 4) << 32) | (1ull << 46);
@@ -770,6 +775,33 @@ __device__ __forceinline__ void wgrad_half(const TcD& T, const TcB& B, const Wgr
     if constexpr (HALF == 0) { conv1(A2{}, r2, o2, b2, w2, hi, lo); conv1(A3{}, r3, o3, b3, w3, hi, lo); }
   };
   const uint32_t id1 = tc_idesc(128, B.N1), id2 = tc_idesc(128, B.N2), id3 = tc_idesc(128, 96);
+  // accumulators -> this CTA's image (added: the image carries the sum over the blocks and launches). Image columns: dW1
+  // [0,N1), dW2 rows 0..127 [N1,N1+N2), rows 128.. [N1+N2,N1+2N2), dW3 [N1+2N2,+96)
+  auto drain = [&]() {  // two 8-column chunks per round: their image loads are in flight together
+    float* dst = a.part + (size_t)blockIdx.x * WG_COLS * 128 + 32 * (warp & 3) + lane;
+    const uint32_t tl = tb + ((uint32_t)(32 * (warp & 3)) << 16);
+    const int ncols = HALF == 0 ? B.N1 + 96 : 2 * B.N2;
+    auto col = [&](int c) { return HALF == 0 ? (c < B.N1 ? c : c + 2 * B.N2) : B.N1 + c; };
+    for (int c0 = 8 * ((warp >> 2) & 1); c0 < ncols; c0 += 32) {
+      const bool two = c0 + 16 < ncols;
+      float v[16], o[16];
+      tmem_ld8(tl + c0, v);
+      if (two) tmem_ld8(tl + c0 + 16, v + 8);
+      const int i0 = col(c0), i1 = col(c0 + 16);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) o[i] = dst[(size_t)(i0 + i) * 128];
+      if (two) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) o[8 + i] = dst[(size_t)(i1 + i) * 128];
+      }
+#pragma unroll
+      for (int i = 0; i < 8; ++i) dst[(size_t)(i0 + i) * 128] = o[i] + v[i];
+      if (two) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) dst[(size_t)(i1 + i) * 128] = o[8 + i] + v[8 + i];
+      }
+    }
+  };
   uint32_t parity[2] = {0u, 0u};
   const int n_mine = blockIdx.x < n_rec ? (n_rec - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
   const int n_sub = 2 * n_mine;
@@ -783,6 +815,14 @@ __device__ __forceinline__ void wgrad_half(const TcD& T, const TcB& B, const Wgr
     float4* lo = hi + set4;
     if (!is_mma) {
       if (u >= 2) { mbar_wait(mbar + b, parity[b]); parity[b] ^= 1u; }  // the MMAs that read this buffer two sub-records ago are done
+      if (u % WG_BLOCK == 0 && u > 0) {
+        // end of an accumulation block: every MMA so far is done (the commit of sub-record u - 1 covers them; the wait of
+        // sub-record u + 1 on the same phase then returns at once); the block's sums go to the image before sub-record u
+        // restarts the accumulators
+        mbar_wait(mbar + (b ^ 1), parity[b ^ 1]);
+        tc_fence_after();
+        drain();
+      }
       convert(hi, lo);
       fence_proxy_async();
       tc_fence_before();
@@ -800,7 +840,7 @@ __device__ __forceinline__ void wgrad_half(const TcD& T, const TcB& B, const Wgr
           const uint32_t sa = pass == 1 ? sl : sh, sb = pass == 0 ? sl : sh;  // hi*lo, lo*hi, hi*hi
 #pragma unroll 1
           for (int s = 0; s < 2; ++s) {
-            const uint32_t acc = (u == 0 && pass == 0 && s == 0) ? 0u : 1u;
+            const uint32_t acc = (u % WG_BLOCK == 0 && pass == 0 && s == 0) ? 0u : 1u;
             auto D = [&](uint32_t base, int off, int rows, int row0) { return wg_desc(base + (uint32_t)(off + 2 * s * rows + row0) * 16, (uint32_t)rows * 16); };
             if constexpr (HALF == 0) {
               tc_mma_ss(tb, D(sa, o0, r0, 0), D(sb, o2, r2, 0), id1, acc);
@@ -822,18 +862,7 @@ __device__ __forceinline__ void wgrad_half(const TcD& T, const TcB& B, const Wgr
     if (n_sub >= 2) { mbar_wait(mbar + (bl ^ 1), parity[bl ^ 1]); }
     mbar_wait(mbar + bl, parity[bl]);
     tc_fence_after();
-    // accumulators -> this CTA's image (added: the image carries the sum over the launches). Image columns: dW1 [0,N1),
-    // dW2 rows 0..127 [N1,N1+N2), rows 128.. [N1+N2,N1+2N2), dW3 [N1+2N2,+96)
-    float* dst = a.part + (size_t)blockIdx.x * WG_COLS * 128;
-    const int qd = warp & 3, part = (warp >> 2) & 1;
-    const int ncols = HALF == 0 ? B.N1 + 96 : 2 * B.N2;
-    for (int c0 = 8 * part; c0 < ncols; c0 += 16) {
-      float v[8];
-      tmem_ld8(tb + ((uint32_t)(32 * qd) << 16) + c0, v);
-      const int ic = HALF == 0 ? (c0 < B.N1 ? c0 : c0 + 2 * B.N2) : B.N1 + c0;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) dst[(size_t)(ic + i) * 128 + 32 * qd + lane] += v[i];
-    }
+    drain();
   }
 }
 
