@@ -304,6 +304,12 @@ int cpz_model_describe(const cpz_model* m, char* buf, size_t buf_len) {
   dump("forward", m->fwd, solve_other_smem(m->desc, m->CT, m->tab.n_stages));
   if (m->has_bwd) dump("adjoint", m->bwd, adjoint_other_smem(m->desc.n_fields * m->desc.Nz, m->desc.n_fields == 3 ? 6 : 2, m->CT));
   else s += "adjoint plan: unavailable (" + m->bwd_err + ")\n";
+  if (m->has_bwd) {
+    snprintf(line, sizeof(line), "rhs pullback (cpz_rhs_vjp): rhs_vjp_kernel, fp32-simt, 32-column tiles on the adjoint plan, weights %s, "
+             "persistent grid of min(tiles, %d) CTAs with one gradient slab each\n",
+             m->bwd.M.w_in_smem ? "in shared memory" : "streamed from global memory", m->ctx->sm_count);
+    s += line;
+  }
   if (m->has_small[0]) {
     const int sms = m->ctx->sm_count > 0 ? m->ctx->sm_count : 148;
     snprintf(line, sizeof(line), "small-batch training pass: 4- / 8- / 16-column adjoint tiles while the batch fits one wave (up to %d / %d / %d columns)\n",
@@ -399,6 +405,74 @@ int cpz_rhs(cpz_model* m, const float* x, const float* bcs, const float* diurnal
   if ((rc = cpz_rhs_dev(m, m->b_x0.p, m->b_bcs.p, diurnal_Q ? m->b_q.p : nullptr, t, m->b_traj.p, ncol))) return rc;
   CPZ_CUDA(cudaMemcpyAsync(dxdt, m->b_traj.p, ncol * S * sizeof(float), cudaMemcpyDeviceToHost, m->ctx->stream));
   CPZ_CUDA(cudaStreamSynchronize(m->ctx->stream));
+  return CPZ_OK;
+}
+
+// ---- RHS pullback ---------------------------------------------------------------------------------------------------
+int cpz_rhs_vjp_dev(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, const float* dxdt_bar,
+                    float* x_bar, float* theta_bar, float* mpp_bar, size_t ncol) {
+  (void)t;  // boundary fluxes, diurnal forcing and t enter f additively: the cotangents do not depend on them
+  int rc = check_model(m);
+  if (rc) return rc;
+  if (ncol == 0) return CPZ_OK;
+  if (!x_bar && !theta_bar && !mpp_bar) return fail(CPZ_ERR_INVALID, "rhs_vjp: no output requested (x_bar, theta_bar and mpp_bar are all NULL)");
+  if (!x || !bcs || !dxdt_bar) return fail(CPZ_ERR_INVALID, "null array");
+  if ((m->desc.flags & CPZ_FLAG_DIURNAL) && !diurnal_Q) return fail(CPZ_ERR_INVALID, "diurnal model needs diurnal_Q");
+  if (theta_bar && m->P == 0) return fail(CPZ_ERR_INVALID, "rhs_vjp: theta_bar requested but the model has no parameters");
+  if (mpp_bar) {  // the checks of cpz_loss_grad_mpp
+    if (m->desc.n_fields != 3) return fail(CPZ_ERR_INVALID, "mPP-parameter gradient needs the u/v/T model");
+    if (!((m->desc.flags & CPZ_FLAG_MPP) || m->desc.variant == CPZ_RHS_INFER)) return fail(CPZ_ERR_INVALID, "mPP-parameter gradient needs CPZ_FLAG_MPP");
+    if (m->desc.flags & CPZ_FLAG_SMOOTH_RI) return fail(CPZ_ERR_INVALID, "mPP-parameter gradient is not available with smooth_Ri");
+  }
+  if (!m->has_bwd) return fail(CPZ_ERR_INVALID, "adjoint plan unavailable: %s", m->bwd_err.c_str());
+  if (ncol > (size_t)INT32_MAX / 512) return fail(CPZ_ERR_INVALID, "ncol too large");
+  if ((rc = bind_device(m->ctx))) return rc;
+  cudaStream_t st = m->ctx->stream;
+  const int P = (int)m->P;
+  const int n_tiles = (int)((ncol + m->CT - 1) / m->CT);
+  const int grid = std::min(n_tiles, m->ctx->sm_count);
+  const size_t slab = (size_t)m->bwd.M.slab;
+  if ((rc = ensure(m->b_part, (size_t)grid * (slab + LP)))) return rc;
+  if ((rc = ensure(m->b_red, (size_t)P + 16))) return rc;
+  float* lpart = m->b_part.p + (size_t)grid * slab;
+  if (theta_bar) CPZ_CUDA(cudaMemsetAsync(m->b_part.p, 0, (size_t)grid * slab * sizeof(float), st));
+  if (mpp_bar) CPZ_CUDA(cudaMemsetAsync(lpart, 0, (size_t)grid * LP * sizeof(float), st));
+  VjpArgs a{};
+  a.theta = m->d_theta; a.x = x; a.ybar = dxdt_bar; a.xbar = x_bar; a.gpart = m->b_part.p; a.lpart = lpart;
+  a.want_mlp = (x_bar || theta_bar) && P > 0; a.want_pgrad = mpp_bar != nullptr; a.ncol = (int)ncol; a.n_tiles = n_tiles;
+  if ((rc = launch_rhs_vjp(m, a, grid))) return rc;
+  if (theta_bar && (rc = launch_reduce_slabs(m, m->b_part.p, grid, P, theta_bar))) return rc;
+  if (mpp_bar) {
+    if ((rc = launch_pack_loss(m, lpart, grid, LP, (float)ncol, m->b_red.p + P))) return rc;
+    CPZ_CUDA(cudaMemcpyAsync(mpp_bar, m->b_red.p + P + 8, 5 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  }
+  return CPZ_OK;
+}
+
+int cpz_rhs_vjp(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, const float* dxdt_bar,
+                float* x_bar, float* theta_bar, float* mpp_bar, size_t ncol) {
+  int rc = check_model(m);
+  if (rc) return rc;
+  if (ncol == 0) return CPZ_OK;
+  if (!x || !bcs || !dxdt_bar) return fail(CPZ_ERR_INVALID, "null array");
+  if ((rc = bind_device(m->ctx))) return rc;
+  if ((rc = upload_inputs(m, x, bcs, diurnal_Q, ncol))) return rc;
+  const size_t S = (size_t)m->fwd.M.S;
+  cudaStream_t st = m->ctx->stream;
+  // staging: ybar in b_tgt, x_bar in b_traj, theta_bar in b_red[0, P) (the pullback's reduction tail is b_red[P, P+16)),
+  // mpp_bar in b_out
+  if ((rc = ensure(m->b_tgt, ncol * S))) return rc;
+  if ((rc = ensure(m->b_traj, ncol * S))) return rc;
+  if ((rc = ensure(m->b_red, m->P + 16))) return rc;
+  if ((rc = ensure(m->b_out, 8))) return rc;
+  CPZ_CUDA(cudaMemcpyAsync(m->b_tgt.p, dxdt_bar, ncol * S * sizeof(float), cudaMemcpyHostToDevice, st));
+  if ((rc = cpz_rhs_vjp_dev(m, m->b_x0.p, m->b_bcs.p, diurnal_Q ? m->b_q.p : nullptr, t, m->b_tgt.p, x_bar ? m->b_traj.p : nullptr,
+                            theta_bar ? m->b_red.p : nullptr, mpp_bar ? m->b_out.p : nullptr, ncol)))
+    return rc;
+  if (x_bar) CPZ_CUDA(cudaMemcpyAsync(x_bar, m->b_traj.p, ncol * S * sizeof(float), cudaMemcpyDeviceToHost, st));
+  if (theta_bar) CPZ_CUDA(cudaMemcpyAsync(theta_bar, m->b_red.p, m->P * sizeof(float), cudaMemcpyDeviceToHost, st));
+  if (mpp_bar) CPZ_CUDA(cudaMemcpyAsync(mpp_bar, m->b_out.p, 5 * sizeof(float), cudaMemcpyDeviceToHost, st));
+  CPZ_CUDA(cudaStreamSynchronize(st));
   return CPZ_OK;
 }
 

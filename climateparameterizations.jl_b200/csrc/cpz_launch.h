@@ -3,6 +3,7 @@
 #include "cpz_internal.h"
 #include "cpz_solve.cuh"
 #include "cpz_adjoint.cuh"
+#include "cpz_rhs_vjp.cuh"
 #include "cpz_closure.cuh"
 #include "cpz_closure_uvt.cuh"
 
@@ -17,6 +18,8 @@ bool closure_uses_tc(const cpz_model* m);  // NN-free u/v/T model; 1 = not eligi
 // one line for cpz_model_describe: which forward kernel this model runs on and why
 std::string tc_describe(const cpz_model* m);  // 1 = not eligible, use the SIMT kernel
 int launch_adjoint(cpz_model* m, const AdjArgs& a, int grid);
+// pullback of one RHS evaluation on the adjoint plan (cpz_k_rhs_vjp.cu): persistent grid, one gradient slab per CTA
+int launch_rhs_vjp(cpz_model* m, const VjpArgs& a, int grid);
 // tensor-core adjoint (cpz_k_adjoint_tc.cu): checkpointing forward solve + reverse sweep; leaves the summed gradient in
 // m->b_red[0,P) and returns the per-tile squared-error sums (stride 8)
 bool adjoint_tc_eligible(cpz_model* m, std::string* why);

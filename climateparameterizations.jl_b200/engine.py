@@ -18,7 +18,7 @@ EXPORTS = [
     "cpz_version", "cpz_last_error", "cpz_device_count", "cpz_sizeof_model_desc", "cpz_sizeof_closure_desc", "cpz_ctx_create", "cpz_ctx_destroy", "cpz_ctx_set_allreduce",
     "cpz_ctx_synchronize", "cpz_ctx_stream", "cpz_ctx_launch_count", "cpz_ctx_nonfinite_count", "cpz_model_create", "cpz_model_destroy",
     "cpz_model_n_params", "cpz_model_n_saved", "cpz_model_describe", "cpz_set_theta", "cpz_get_theta", "cpz_model_set_time", "cpz_rhs",
-    "cpz_rhs_dev", "cpz_predict_flux", "cpz_predict_flux_dev", "cpz_solve", "cpz_solve_dev", "cpz_loss_grad", "cpz_loss_grad_dev", "cpz_train_step",
+    "cpz_rhs_dev", "cpz_rhs_vjp", "cpz_rhs_vjp_dev", "cpz_predict_flux", "cpz_predict_flux_dev", "cpz_solve", "cpz_solve_dev", "cpz_loss_grad", "cpz_loss_grad_dev", "cpz_train_step",
     "cpz_train_step_dev", "cpz_set_mpp_params", "cpz_get_mpp_params", "cpz_loss_grad_mpp", "cpz_loss_grad_mpp_dev", "cpz_adam_get_state", "cpz_adam_set_state", "cpz_closure_step", "cpz_closure_step_dev",
     "cpz_sizeof_closure_uvt_desc", "cpz_closure_step_uvt", "cpz_closure_step_uvt_dev",
 ]
@@ -68,6 +68,8 @@ def lib() -> C.CDLL:
     L.cpz_model_set_time.argtypes = [vp, i32, f32, f32, i32, i32, i32, i32]
     for name in ("cpz_rhs", "cpz_rhs_dev", "cpz_predict_flux", "cpz_predict_flux_dev"):
         getattr(L, name).argtypes = [vp, vp, vp, vp, f32, vp, sz]
+    for name in ("cpz_rhs_vjp", "cpz_rhs_vjp_dev"):
+        getattr(L, name).argtypes = [vp, vp, vp, vp, f32, vp, vp, vp, vp, sz]
     for name in ("cpz_solve", "cpz_solve_dev"):
         getattr(L, name).argtypes = [vp, vp, vp, vp, vp, sz]
     for name in ("cpz_loss_grad", "cpz_loss_grad_dev"):
@@ -246,6 +248,22 @@ class Model:
         _check(lib().cpz_rhs(self._h, _ptr(x), _ptr(bcs), _ptr(Q), float(t), _ptr(out), ncol))
         return out
 
+    def rhs_vjp(self, x, bcs, dxdt_bar, t: float = 0.0, Q=None, want_x: bool = True, want_theta: bool = True,
+                want_mpp: bool = False):
+        """Pullback of rhs() at x for the cotangent dxdt_bar [ncol, S] — cpz_rhs_vjp. Returns (x_bar [ncol, S],
+        theta_bar [P], mpp_bar [5] wrt (nu0, nu_m, dRi, Ric, Pr)); an output that is not wanted is None."""
+        x = _np(x)
+        ncol = x.shape[0]
+        bcs = _np(bcs, (ncol, self.desc.n_bc))
+        ybar = _np(dxdt_bar, x.shape)
+        Q = None if Q is None else _np(Q, (ncol,))
+        xb = np.empty_like(x) if want_x else None
+        tb = np.empty(self.P, dtype=np.float32) if want_theta else None
+        pb = np.empty(5, dtype=np.float32) if want_mpp else None
+        _check(lib().cpz_rhs_vjp(self._h, _ptr(x), _ptr(bcs), _ptr(Q), float(t), _ptr(ybar), _ptr(xb), _ptr(tb), _ptr(pb),
+                                 ncol))
+        return xb, tb, pb
+
     def predict_flux(self, x, bcs, t: float = 0.0, Q=None) -> np.ndarray:
         """Total face fluxes [ncol, n_fields, Nz+1] (scaled) of one RHS evaluation — cpz_predict_flux."""
         x = _np(x)
@@ -356,6 +374,13 @@ class Model:
     def rhs_dev(self, x, bcs, out, t: float = 0.0, Q=None, ncol: Optional[int] = None) -> None:
         ncol = ncol if ncol is not None else x.shape[0]
         _check(lib().cpz_rhs_dev(self._h, _ptr(x), _ptr(bcs), _ptr(Q), float(t), _ptr(out), ncol))
+
+    def rhs_vjp_dev(self, x, bcs, dxdt_bar, x_bar=None, theta_bar=None, mpp_bar=None, t: float = 0.0, Q=None,
+                    ncol: Optional[int] = None) -> None:
+        """cpz_rhs_vjp_dev: the outputs given (x_bar [ncol, S], theta_bar [P], mpp_bar [5]) are overwritten."""
+        ncol = ncol if ncol is not None else x.shape[0]
+        _check(lib().cpz_rhs_vjp_dev(self._h, _ptr(x), _ptr(bcs), _ptr(Q), float(t), _ptr(dxdt_bar), _ptr(x_bar),
+                                     _ptr(theta_bar), _ptr(mpp_bar), ncol))
 
     def solve_dev(self, x0, bcs, traj, Q=None, ncol: Optional[int] = None) -> None:
         ncol = ncol if ncol is not None else x0.shape[0]

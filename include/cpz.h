@@ -177,6 +177,24 @@ int cpz_model_set_time(cpz_model* m, int32_t integrator, float dt, float t0, int
 int cpz_rhs(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, float* dxdt, size_t ncol);
 int cpz_rhs_dev(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, float* dxdt, size_t ncol);
 
+/* ---- S1 pullback: VJP of f(x, p, t) ------------------------------------------------------------ */
+/* replaces the Zygote pullback of NDE that InterpolatingAdjoint(autojacvec=ZygoteVJP()) calls once per adjoint stage
+ * (NDE_training.jl:291,304; free_convection/src/solve.jl:4-5), so that a host with its own time stepper (adaptive Tsit5 or
+ * ROCK4, a continuous adjoint) can differentiate through cpz_rhs. With f_c = what cpz_rhs returns for column c on the same
+ * inputs and ybar_c = dxdt_bar[c] ([ncol][nf*Nz]):
+ *   x_bar[c]  = (df_c/dx_c)^T ybar_c                 [ncol][nf*Nz]
+ *   theta_bar = sum_c (df_c/dtheta)^T ybar_c         [P], Flux.destructure order
+ *   mpp_bar   = sum_c (df_c/dp)^T ybar_c             [5], p = (nu0, nu_m, dRi, Ric, Pr) unscaled, as cpz_loss_grad_mpp
+ * Outputs are overwritten, not accumulated; each may be NULL, at least one must not be. theta_bar must be NULL when P = 0;
+ * mpp_bar is refused where cpz_loss_grad_mpp refuses it. At relu kinks and the convective-adjustment switch the derivative
+ * of the branch that was evaluated is taken. With CPZ_FLAG_IMPLICIT_DIFFUSION this is the pullback of the explicit part
+ * cpz_rhs returns (mpp_bar = 0). The sums over columns are in a fixed order (bitwise reproducible); the allreduce hook is
+ * not called (the sum over ranks is the host's) and there is no non-finite reporting. Needs the adjoint plan. */
+int cpz_rhs_vjp(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, const float* dxdt_bar,
+                float* x_bar, float* theta_bar, float* mpp_bar, size_t ncol);
+int cpz_rhs_vjp_dev(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, const float* dxdt_bar,
+                    float* x_bar, float* theta_bar, float* mpp_bar, size_t ncol);
+
 /* total face fluxes of one RHS evaluation; replaces predict_flux (NDE_training.jl:83-147), predict_flux! (training_postprocessing.jl:
  * 105-128) and the per-frame wT reconstruction of solve_nde (free_convection/src/solve.jl:35-48).
  * flux: [ncol][n_fields][Nz+1] (scaled): faces 0 and Nz are the effective boundary fluxes, interior faces NN flux minus the
