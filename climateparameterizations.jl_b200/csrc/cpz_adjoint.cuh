@@ -30,6 +30,8 @@ struct AdjArgs {
   float w[6];
   float inv_prof, inv_grad;  // 1/(Nz*n_saved*ncol_global), 1/((Nz+1)*n_saved*ncol_global)
   unsigned long long* prof;  // optional [8] cycle counters of CTA 0 (CPZ_PROF=1)
+  const float* cot;      // [ncol][n_saved][S] cotangent of the trajectory (cpz_solve_vjp): selects adjoint_kernel<..., true>
+  float* x0bar;          // [ncol][S] cotangent of x0 (cot mode), or null
 };
 #define CPZ_APROF_T() ((a.prof && blockIdx.x == 0 && threadIdx.x == 0) ? clock64() : 0)
 #define CPZ_APROF_ADD(slot, t0) do { if (a.prof && blockIdx.x == 0 && threadIdx.x == 0) a.prof[slot] += (unsigned long long)(clock64() - (t0)); } while (0)
@@ -479,6 +481,15 @@ __device__ __noinline__ void loss_frame(const ModelD& M, const AdjArgs& a, const
   }
 }
 
+// cot mode (cpz_solve_vjp): the trajectory cotangent of one saved frame, cb (a tile loaded like the targets), goes into
+// xbar unchanged. load_tile replicates the last valid column into the padding columns, which must stay at zero.
+template <int CT, int NT>
+__device__ __noinline__ void cot_frame(const ModelD& M, const float* __restrict__ cb, float* __restrict__ xbar, int nvalid) {
+  for (int it = threadIdx.x; it < M.S * CT; it += NT) {
+    if (it % CT < nvalid) xbar[it] += cb[it];
+  }
+}
+
 // Global arrays shared with the forward kernels (checkpoints, stored stage tendencies) are laid out in 32-column tiles
 // [tile32][...][S][32] whatever this kernel's tile width CT is (CT divides 32): float4 number e4 of a [S][CT] tile sits at
 // row e4 / (CT/4), float4 e4 % (CT/4) of a row of `ld` floats. The CTA's private scratch uses ld = CT (contiguous).
@@ -621,7 +632,9 @@ __device__ __noinline__ void implicit_vjp_tile(const ModelD& M, const float* __r
   }
 }
 
-template <int CT, int NT, bool WS, int NF>
+// COT: cot mode (cpz_solve_vjp) — the trajectory cotangent a.cot replaces the loss terms at the saved frames and the
+// cotangent of x0 is stored to a.x0bar. A template parameter so that the loss-mode kernels are compiled as before.
+template <int CT, int NT, bool WS, int NF, bool COT>
 __device__ __forceinline__ void adjoint_body(const ModelD& M, const ModelD& Mp, const TableauD& tab, const TimeD& tm,
                                              const AdjArgs& a, float* smem) {
   const AdjSmem L = adjoint_smem_layout(M, CT);
@@ -690,9 +703,10 @@ __device__ __forceinline__ void adjoint_body(const ModelD& M, const ModelD& Mp, 
     {
       const int fr = frame_of(tm.n_steps);
       if (fr >= 0) {
-        load_tile<CT, NT>(xb, xin, bar, parity, a.targets + (size_t)fr * S, (size_t)a.n_saved * S, S, col0, a.ncol);
+        load_tile<CT, NT>(xb, xin, bar, parity, (COT ? a.cot : a.targets) + (size_t)fr * S, (size_t)a.n_saved * S, S, col0, a.ncol);
         __syncthreads();
-        loss_frame<CT, NT>(M, a, xs, xb, xbar, nvalid, lsum);
+        if constexpr (COT) cot_frame<CT, NT>(M, xb, xbar, nvalid);
+        else loss_frame<CT, NT>(M, a, xs, xb, xbar, nvalid, lsum);
         __syncthreads();
       }
     }
@@ -835,15 +849,22 @@ __device__ __forceinline__ void adjoint_body(const ModelD& M, const ModelD& Mp, 
         if (sub == 0) {
           const int fr = frame_of(nstep);
           if (fr >= 0) {
-            load_tile<CT, NT>(xb, xin, bar, parity, a.targets + (size_t)fr * S, (size_t)a.n_saved * S, S, col0, a.ncol);
+            load_tile<CT, NT>(xb, xin, bar, parity, (COT ? a.cot : a.targets) + (size_t)fr * S, (size_t)a.n_saved * S, S, col0, a.ncol);
             __syncthreads();
-            loss_frame<CT, NT>(M, a, xs, xb, xbar, nvalid, lsum);
+            if constexpr (COT) cot_frame<CT, NT>(M, xb, xbar, nvalid);
+            else loss_frame<CT, NT>(M, a, xs, xb, xbar, nvalid, lsum);
             __syncthreads();
           }
         }
       }
     }
+    if (COT && a.x0bar != nullptr) {  // xbar is now the cotangent of x0
+      __syncthreads();
+      store_tile<CT, NT>(xbar, xin, a.x0bar, (size_t)S, S, col0, a.ncol);
+      if (threadIdx.x < CT) bulk_wait_read0();  // xin is the next tile's staging buffer
+    }
   }
+  if (COT && a.x0bar != nullptr && threadIdx.x < CT) bulk_wait0();
   // block reduction of the six loss sums and the five mPP-parameter gradient sums
   for (int q = 0; q < 11; ++q) {
     double vd = q < 6 ? (double)lsum[q] : pgs[q - 6];
@@ -860,14 +881,14 @@ __device__ __forceinline__ void adjoint_body(const ModelD& M, const ModelD& Mp, 
   }
 }
 
-template <int CT, int NT, bool WS>
+template <int CT, int NT, bool WS, bool COT>
 __global__ void __launch_bounds__(NT, 1) adjoint_kernel(const __grid_constant__ ModelD Mp, const __grid_constant__ TableauD tab,
                                                         const TimeD tm, const __grid_constant__ AdjArgs a) {
   extern __shared__ __align__(16) float smem[];
   const AdjSmem L = adjoint_smem_layout(Mp, CT);
   const ModelD& M = model_to_smem<NT>(Mp, smem + L.model);
-  if (Mp.nf == 3) adjoint_body<CT, NT, WS, 3>(M, Mp, tab, tm, a, smem);
-  else adjoint_body<CT, NT, WS, 1>(M, Mp, tab, tm, a, smem);
+  if (Mp.nf == 3) adjoint_body<CT, NT, WS, 3, COT>(M, Mp, tab, tm, a, smem);
+  else adjoint_body<CT, NT, WS, 1, COT>(M, Mp, tab, tm, a, smem);
 }
 
 struct W6 { float w[6]; };

@@ -1,4 +1,4 @@
-// Launcher of adjoint_kernel<CT,NT,WS> shared by the 32-column (cpz_k_adjoint.cu) and small-tile (cpz_k_small.cu) translation units.
+// Launcher of adjoint_kernel<CT,NT,WS,COT> shared by the 32-column (cpz_k_adjoint.cu) and small-tile (cpz_k_small.cu) translation units.
 #pragma once
 #include <cstdio>
 #include <cstdlib>
@@ -12,7 +12,7 @@ static int launch_adjoint_t(cpz_model* m, const Plan& plan, const AdjArgs& a, in
   const AdjSmem L = adjoint_smem_layout(plan.M, CT);
   const size_t smem = (size_t)L.total_floats * sizeof(float);
   if (smem > m->ctx->smem_optin) return fail(CPZ_ERR_INVALID, "adjoint kernel needs %zu B shared memory, device allows %zu", smem, m->ctx->smem_optin);
-  auto kern = adjoint_kernel<CT, NT, WS>;
+  auto kern = a.cot != nullptr ? adjoint_kernel<CT, NT, WS, true> : adjoint_kernel<CT, NT, WS, false>;
   CPZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   static const bool prof = getenv("CPZ_PROF") != nullptr;
   if (prof) {

@@ -94,6 +94,8 @@ struct AdjTcArgs {
   int seg_step0, seg_steps;
   float w[6];
   float inv_prof, inv_grad;
+  const float* cot;      // [ncol][n_saved][96] cotangent of the trajectory (cpz_solve_vjp): selects adjoint_tc_kernel<..., true>
+  float* x0bar;          // [ncol][96] cotangent of x0, written by the launch that ends at step 0 (cot mode), or null
 };
 
 constexpr int TCB_SIDE_ARRAYS = 11;  // X_u X_v X_T | e_u e_v e_T (face-flux cotangents) | g_u g_v g_T (cotangents of the level differences) | kbar_u kbar_v
@@ -167,7 +169,8 @@ __device__ __forceinline__ void side_column_vjp(const SideC& C, float du, float 
 
 // ---- reverse sweep over one checkpoint segment -----------------------------------------------------------------------
 // IMPL: CPZ_FLAG_IMPLICIT_DIFFUSION models (the VJP of the implicit step is compiled only into this instantiation)
-template <int ACT, bool IMPL = false>
+// COT: cot mode (cpz_solve_vjp): a.cot replaces the loss terms; a template parameter because the kernel has no register headroom
+template <int ACT, bool IMPL = false, bool COT = false>
 __global__ void __launch_bounds__(TC_NT, 1) adjoint_tc_kernel(const __grid_constant__ ModelD M, const __grid_constant__ TcD T,
                                                               const __grid_constant__ TcB B, const __grid_constant__ TableauD tab,
                                                               const TimeD tm, const __grid_constant__ AdjTcArgs a) {
@@ -227,6 +230,16 @@ __global__ void __launch_bounds__(TC_NT, 1) adjoint_tc_kernel(const __grid_const
   const float Nf = M.rc.Nf;
   // loss terms of one saved frame at state xs (loss.jl:1-42): squared-error sums and d(loss)/dx into xbar
   auto loss_frame = [&](const float* xs, int fr) {
+    if constexpr (COT) {  // the trajectory cotangent of the frame, 0 on padding columns
+      if (qd < 3) {
+#pragma unroll
+        for (int r = 0; r < 8; ++r) {
+          const int col = col0 + cg0 + r;
+          if (col < a.ncol) xbar[r] += __ldg(a.cot + ((size_t)col * a.n_saved + fr) * 96 + 32 * qd + lane);
+        }
+      }
+      return;
+    }
     if (qd < 3) {
 #pragma unroll
       for (int r = 0; r < 8; ++r) {
@@ -615,6 +628,13 @@ __global__ void __launch_bounds__(TC_NT, 1) adjoint_tc_kernel(const __grid_const
   if (qd < 3 && active) {
     reinterpret_cast<float4*>(xb_g)[0] = make_float4(xbar[0], xbar[1], xbar[2], xbar[3]);
     reinterpret_cast<float4*>(xb_g)[1] = make_float4(xbar[4], xbar[5], xbar[6], xbar[7]);
+    if (COT && a.x0bar != nullptr) {
+#pragma unroll
+      for (int r = 0; r < 8; ++r) {
+        const int col = col0 + cg0 + r;
+        if (col < a.ncol) a.x0bar[(size_t)col * 96 + 32 * qd + lane] = xbar[r];
+      }
+    }
   }
   // squared-error sums: fixed-order reduction (warp shuffles, then the six sums over the warps of a field)
   for (int o = 16; o > 0; o >>= 1) { lp += __shfl_xor_sync(0xffffffffu, lp, o); lg += __shfl_xor_sync(0xffffffffu, lg, o); }

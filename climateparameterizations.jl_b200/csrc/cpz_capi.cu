@@ -310,6 +310,8 @@ int cpz_model_describe(const cpz_model* m, char* buf, size_t buf_len) {
              m->bwd.M.w_in_smem ? "in shared memory" : "streamed from global memory", m->ctx->sm_count);
     s += line;
   }
+  s += "solve pullback (cpz_solve_vjp): the cpz_loss_grad kernels above in cotangent mode (the trajectory cotangent replaces the "
+       "loss terms at the saved frames; x0 cotangent stored at the end of the reverse sweep)\n";
   if (m->has_small[0]) {
     const int sms = m->ctx->sm_count > 0 ? m->ctx->sm_count : 148;
     snprintf(line, sizeof(line), "small-batch training pass: 4- / 8- / 16-column adjoint tiles while the batch fits one wave (up to %d / %d / %d columns)\n",

@@ -43,6 +43,8 @@ struct Fc1Args {
   float* lpart;          // [ncol][8]: squared-error sum of the T profiles at index 2
   int ncol, n_saved, n_sub;  // n_sub = n_steps * n_substeps
   float wT, inv_prof;
+  const float* cot;      // [ncol][n_saved][32] cotangent of the trajectory (cpz_solve_vjp), or null: loss mode (targets)
+  float* x0bar;          // [ncol][32] cotangent of x0 (cot mode), or null
 };
 
 // zero-padded weight copy in shared memory
@@ -270,6 +272,10 @@ __global__ void __launch_bounds__(FC1_NT, 1) fc1_train_kernel(const __grid_const
   };
   float sse = 0.f;
   auto loss_frame = [&](const float* __restrict__ x, int fr) {  // warp 0
+    if (a.cot != nullptr) {
+      xbar[lane] += __ldg(a.cot + ((size_t)col * a.n_saved + fr) * 32 + lane);
+      return;
+    }
     const float d = x[lane] - __ldg(a.targets + ((size_t)col * a.n_saved + fr) * 32 + lane);
     sse = fmaf(d, d, sse);
     xbar[lane] += a.wT * 2.f * a.inv_prof * d;
@@ -429,7 +435,9 @@ __global__ void __launch_bounds__(FC1_NT, 1) fc1_train_kernel(const __grid_const
         if (r % nsub == 0) {
           const int fr = frame_of(r / nsub);
           if (fr >= 0) {
-            if (implicit) {  // the saved frame is the state before the step's first implicit solve
+            if (a.cot != nullptr) {
+              xbar[lane] += __ldg(a.cot + ((size_t)col * a.n_saved + fr) * 32 + lane);
+            } else if (implicit) {  // the saved frame is the state before the step's first implicit solve
               const float d = xp_cur - __ldg(a.targets + ((size_t)col * a.n_saved + fr) * 32 + lane);
               sse = fmaf(d, d, sse);
               xbar[lane] += a.wT * 2.f * a.inv_prof * d;
@@ -464,6 +472,7 @@ __global__ void __launch_bounds__(FC1_NT, 1) fc1_train_kernel(const __grid_const
   if (t < 32) {
     for (int o = 16; o > 0; o >>= 1) sse += __shfl_xor_sync(0xffffffffu, sse, o);
     if (t < 8) a.lpart[(size_t)col * 8 + t] = t == 2 ? sse : 0.f;
+    if (a.x0bar != nullptr) a.x0bar[(size_t)col * 32 + lane] = xbar[lane];
   }
 }
 

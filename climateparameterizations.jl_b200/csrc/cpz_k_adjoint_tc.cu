@@ -47,7 +47,9 @@ template <int ACT>
 static int launch_reverse_t(cpz_model* m, const TcD& T, const TcB& B, const AdjTcArgs& aa, const TimeD& tm, int n_ctas, const WgradArgs& wa,
                             int wg_grid, size_t wg_smem, bool ref) {
   const TcBSmem L = tc_bwd_smem_layout(B, m->tab.n_stages);
-  auto kern = (m->desc.flags & CPZ_FLAG_IMPLICIT_DIFFUSION) ? adjoint_tc_kernel<ACT, true> : adjoint_tc_kernel<ACT, false>;
+  const bool impl = (m->desc.flags & CPZ_FLAG_IMPLICIT_DIFFUSION) != 0;
+  auto kern = aa.cot != nullptr ? (impl ? adjoint_tc_kernel<ACT, true, true> : adjoint_tc_kernel<ACT, false, true>)
+                                : (impl ? adjoint_tc_kernel<ACT, true, false> : adjoint_tc_kernel<ACT, false, false>);
   CPZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
   kern<<<n_ctas, TC_NT, L.total, m->ctx->stream>>>(m->fwd.M, T, B, m->tab, tm, aa);
   CPZ_CUDA(cudaGetLastError());
@@ -73,7 +75,8 @@ static int launch_reverse_t(cpz_model* m, const TcD& T, const TcB& B, const AdjT
 // On return m->b_red[0,P) holds the sum over the local columns of d(unnormalised loss)/dtheta and *lpart_out / *n_lpart the
 // per-tile squared-error sums (stride 8).
 int loss_grad_tc(cpz_model* m, const float* x0, const float* bcs, const float* Q, const float* targets, size_t ncol,
-                 const float* loss_w, float inv_prof, float inv_grad, int n_saved, int n_ckpt, const float** lpart_out, int* n_lpart) {
+                 const float* loss_w, float inv_prof, float inv_grad, int n_saved, int n_ckpt, const float** lpart_out, int* n_lpart,
+                 CotPair cp) {
   TcD T;
   TcB B;
   std::string why;
@@ -192,7 +195,8 @@ int loss_grad_tc(cpz_model* m, const float* x0, const float* bcs, const float* Q
     for (int n1 = a1; n1 > a0; n1 -= std::min(rs, n1 - a0)) {
       const int n0 = n1 - std::min(rs, n1 - a0);
       AdjTcArgs aa{};
-      aa.wimg = m->b_bwimg.p; aa.theta = m->d_theta; aa.targets = targets;
+      aa.wimg = m->b_bwimg.p; aa.theta = m->d_theta; aa.targets = targets; aa.cot = cp.cot;
+      aa.x0bar = n0 == 0 ? cp.x0bar : nullptr;  // the launch that ends the reverse sweep at step 0
       aa.xN = m->b_ckpt.p + (size_t)(n_ckpt - 1) * SL; aa.xN_stride = (size_t)n_ckpt * SL;
       aa.xbar = xbar; aa.lpart = lpart; aa.aux = A;
       aa.aux.ev0 = (n0 - a0) * epst;

@@ -55,7 +55,7 @@ bool fc1_eligible(const cpz_model* m, size_t ncol) {
 // Leaves the sum over the columns of d(unnormalised loss)/dtheta in m->b_red[0,P) and returns the per-column squared-error
 // sums (stride 8).
 int loss_grad_fc1(cpz_model* m, const float* x0, const float* bcs, const float* targets, size_t ncol, float wT, float inv_prof,
-                  int n_saved, const float** lpart_out) {
+                  int n_saved, const float** lpart_out, CotPair cp) {
   Fc1D F;
   if (!fc1_plan(m, F)) return fail(CPZ_ERR_INVALID, "single-column training kernel not eligible");
   const int P = F.P;
@@ -66,7 +66,7 @@ int loss_grad_fc1(cpz_model* m, const float* x0, const float* bcs, const float* 
   const bool implicit = (m->desc.flags & CPZ_FLAG_IMPLICIT_DIFFUSION) != 0;
   if (implicit && (rc = fc1_ensure(m->b_scr, ncol * (size_t)n_sub * 32))) return rc;
   Fc1Args a{};
-  a.theta = m->d_theta; a.x0 = x0; a.x0_stride = 0; a.bcs = bcs; a.targets = targets;
+  a.theta = m->d_theta; a.x0 = x0; a.x0_stride = 0; a.bcs = bcs; a.targets = targets; a.cot = cp.cot; a.x0bar = cp.x0bar;
   a.records = m->b_ckpt.p; a.xp = implicit ? m->b_scr.p : nullptr; a.gpart = m->b_part.p; a.lpart = m->b_part.p + ncol * (size_t)P;
   a.ncol = (int)ncol; a.n_saved = n_saved; a.n_sub = n_sub; a.wT = wT; a.inv_prof = inv_prof;
   const Fc1Smem L = fc1_smem_layout(m->tab.n_stages);

@@ -8,6 +8,12 @@
 #include "cpz_closure_uvt.cuh"
 
 namespace cpz {
+// cotangent mode of the training pass (cpz_solve_vjp): the [ncol][n_saved][S] trajectory cotangent replaces the loss terms
+// at every saved frame, and x0bar ([ncol][S], may be null) receives the cotangent of x0. cot == nullptr: loss mode.
+struct CotPair {
+  const float* cot = nullptr;
+  float* x0bar = nullptr;
+};
 int launch_solve(cpz_model* m, const SolveArgs& a);
 int launch_flux(cpz_model* m, const SolveArgs& a);  // rhs_only == 2 on the FP32 kernel with the adjoint plan's face-flux rows
 int launch_solve_tc(cpz_model* m, const SolveArgs& a);
@@ -24,7 +30,8 @@ int launch_rhs_vjp(cpz_model* m, const VjpArgs& a, int grid);
 // m->b_red[0,P) and returns the per-tile squared-error sums (stride 8)
 bool adjoint_tc_eligible(cpz_model* m, std::string* why);
 int loss_grad_tc(cpz_model* m, const float* x0, const float* bcs, const float* Q, const float* targets, size_t ncol,
-                 const float* loss_w, float inv_prof, float inv_grad, int n_saved, int n_ckpt, const float** lpart_out, int* n_lpart);
+                 const float* loss_w, float inv_prof, float inv_grad, int n_saved, int n_ckpt, const float** lpart_out, int* n_lpart,
+                 CotPair cp = CotPair{});
 // 4-, 8- and 16-column-tile instantiations (cpz_k_small.cu, cpz_k_small8.cu, cpz_k_small16.cu); CT selects the plan
 int launch_solve_small(cpz_model* m, const SolveArgs& a, int CT);
 int launch_adjoint_small(cpz_model* m, const AdjArgs& a, int grid, int CT);
@@ -33,7 +40,7 @@ int train_tile(const cpz_model* m, size_t ncol);
 // small-batch T-only training pass, one CTA per column (cpz_k_fc1.cu)
 bool fc1_eligible(const cpz_model* m, size_t ncol);
 int loss_grad_fc1(cpz_model* m, const float* x0, const float* bcs, const float* targets, size_t ncol, float wT, float inv_prof,
-                  int n_saved, const float** lpart_out);
+                  int n_saved, const float** lpart_out, CotPair cp = CotPair{});
 int launch_closure(cpz_model* m, const ClosureD& cd, const ClosureArgs& a);
 int launch_closure_uvt(cpz_model* m, const ClosureUvtD& cd, const ClosureUvtArgs& a);
 int launch_closure_uvt_tc(cpz_model* m, const ClosureUvtD& cd, const ClosureUvtArgs& a);  // tcgen05 flavour (cpz_k_tc.cu); 1 = not eligible

@@ -18,7 +18,7 @@ EXPORTS = [
     "cpz_version", "cpz_last_error", "cpz_device_count", "cpz_sizeof_model_desc", "cpz_sizeof_closure_desc", "cpz_ctx_create", "cpz_ctx_destroy", "cpz_ctx_set_allreduce",
     "cpz_ctx_synchronize", "cpz_ctx_stream", "cpz_ctx_launch_count", "cpz_ctx_nonfinite_count", "cpz_model_create", "cpz_model_destroy",
     "cpz_model_n_params", "cpz_model_n_saved", "cpz_model_describe", "cpz_set_theta", "cpz_get_theta", "cpz_model_set_time", "cpz_rhs",
-    "cpz_rhs_dev", "cpz_rhs_vjp", "cpz_rhs_vjp_dev", "cpz_predict_flux", "cpz_predict_flux_dev", "cpz_solve", "cpz_solve_dev", "cpz_loss_grad", "cpz_loss_grad_dev", "cpz_train_step",
+    "cpz_rhs_dev", "cpz_rhs_vjp", "cpz_rhs_vjp_dev", "cpz_predict_flux", "cpz_predict_flux_dev", "cpz_solve", "cpz_solve_dev", "cpz_solve_vjp", "cpz_solve_vjp_dev", "cpz_loss_grad", "cpz_loss_grad_dev", "cpz_train_step",
     "cpz_train_step_dev", "cpz_set_mpp_params", "cpz_get_mpp_params", "cpz_loss_grad_mpp", "cpz_loss_grad_mpp_dev", "cpz_adam_get_state", "cpz_adam_set_state", "cpz_closure_step", "cpz_closure_step_dev",
     "cpz_sizeof_closure_uvt_desc", "cpz_closure_step_uvt", "cpz_closure_step_uvt_dev",
 ]
@@ -72,6 +72,8 @@ def lib() -> C.CDLL:
         getattr(L, name).argtypes = [vp, vp, vp, vp, f32, vp, vp, vp, vp, sz]
     for name in ("cpz_solve", "cpz_solve_dev"):
         getattr(L, name).argtypes = [vp, vp, vp, vp, vp, sz]
+    for name in ("cpz_solve_vjp", "cpz_solve_vjp_dev"):
+        getattr(L, name).argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, sz]
     for name in ("cpz_loss_grad", "cpz_loss_grad_dev"):
         getattr(L, name).argtypes = [vp, vp, vp, vp, vp, sz, vp, vp, vp]
     for name in ("cpz_loss_grad_mpp", "cpz_loss_grad_mpp_dev"):
@@ -284,6 +286,20 @@ class Model:
         _check(lib().cpz_solve(self._h, _ptr(x0), _ptr(bcs), _ptr(Q), _ptr(out), ncol))
         return out
 
+    def solve_vjp(self, x0, bcs, traj_bar, Q=None, want_x0: bool = True, want_theta: bool = True, want_mpp: bool = False):
+        """Pullback of solve() at x0 for the cotangent traj_bar [ncol, n_saved, S] — cpz_solve_vjp. Returns (x0_bar
+        [ncol, S], theta_bar [P], mpp_bar [5] wrt (nu0, nu_m, dRi, Ric, Pr)); an output that is not wanted is None."""
+        x0 = _np(x0)
+        ncol = x0.shape[0]
+        bcs = _np(bcs, (ncol, self.desc.n_bc))
+        tb_in = _np(traj_bar, (ncol, self.n_saved, self.desc.S))
+        Q = None if Q is None else _np(Q, (ncol,))
+        xb = np.empty_like(x0) if want_x0 else None
+        tb = np.empty(self.P, dtype=np.float32) if want_theta else None
+        pb = np.empty(5, dtype=np.float32) if want_mpp else None
+        _check(lib().cpz_solve_vjp(self._h, _ptr(x0), _ptr(bcs), _ptr(Q), _ptr(tb_in), _ptr(xb), _ptr(tb), _ptr(pb), ncol))
+        return xb, tb, pb
+
     def loss_grad(self, x0, bcs, targets, loss_w, Q=None, want_grad: bool = True):
         x0 = _np(x0)
         ncol = x0.shape[0]
@@ -385,6 +401,13 @@ class Model:
     def solve_dev(self, x0, bcs, traj, Q=None, ncol: Optional[int] = None) -> None:
         ncol = ncol if ncol is not None else x0.shape[0]
         _check(lib().cpz_solve_dev(self._h, _ptr(x0), _ptr(bcs), _ptr(Q), _ptr(traj), ncol))
+
+    def solve_vjp_dev(self, x0, bcs, traj_bar, x0_bar=None, theta_bar=None, mpp_bar=None, Q=None,
+                      ncol: Optional[int] = None) -> None:
+        """cpz_solve_vjp_dev: the outputs given (x0_bar [ncol, S], theta_bar [P], mpp_bar [5]) are overwritten."""
+        ncol = ncol if ncol is not None else x0.shape[0]
+        _check(lib().cpz_solve_vjp_dev(self._h, _ptr(x0), _ptr(bcs), _ptr(Q), _ptr(traj_bar), _ptr(x0_bar), _ptr(theta_bar),
+                                       _ptr(mpp_bar), ncol))
 
     def loss_grad_dev(self, x0, bcs, targets, loss_w, loss_out, grad_out, Q=None, ncol: Optional[int] = None) -> None:
         ncol = ncol if ncol is not None else x0.shape[0]

@@ -209,6 +209,27 @@ int cpz_predict_flux_dev(cpz_model* m, const float* x, const float* bcs, const f
 int cpz_solve(cpz_model* m, const float* x0, const float* bcs, const float* diurnal_Q, float* traj, size_t ncol);
 int cpz_solve_dev(cpz_model* m, const float* x0, const float* bcs, const float* diurnal_Q, float* traj, size_t ncol);
 
+/* ---- S2 pullback: VJP of the solve ---------------------------------------------------------------------------------- */
+/* replaces the Zygote pullback of Array(solve(prob, ...; sensealg = InterpolatingAdjoint(...))) that loss_NDE /
+ * loss_gradient_NDE (NDE_training.jl:290-323) and nde_loss (free_convection/src/training.jl:55-62) take of the loss they
+ * compute on the trajectory, so that a host can differentiate any loss of the solve, not only cpz_loss_grad's. With
+ * traj_c = what cpz_solve writes for column c on the same inputs (current theta, mPP parameters and time settings) and
+ * tbar_c = traj_bar[c] ([ncol][n_saved][nf*Nz], the layout of traj and targets):
+ *   x0_bar[c] = (dtraj_c/dx0_c)^T tbar_c             [ncol][nf*Nz]; frame 0 is x0 itself when save_stride > 0
+ *   theta_bar = sum_c (dtraj_c/dtheta)^T tbar_c      [P], Flux.destructure order
+ *   mpp_bar   = sum_c (dtraj_c/dp)^T tbar_c          [5], p = (nu0, nu_m, dRi, Ric, Pr) unscaled, as cpz_loss_grad_mpp
+ * This is the exact discrete adjoint of the engine's fixed-step map, computed by cpz_loss_grad's kernels (checkpointing
+ * forward, then the reverse sweep) with traj_bar in place of the loss terms; kinks are handled as there. Outputs are
+ * overwritten, not accumulated; each may be NULL, at least one must not be. theta_bar must be NULL when P = 0; mpp_bar is
+ * refused where cpz_loss_grad_mpp refuses it, and an implicit-diffusion model where cpz_loss_grad refuses it. The sums
+ * over columns are in a fixed order; the allreduce hook is not called (the sum over ranks is the host's) and there is no
+ * non-finite reporting. The argument checks are cpz_loss_grad's with traj_bar in place of targets; the device scratch is
+ * cpz_loss_grad's. */
+int cpz_solve_vjp(cpz_model* m, const float* x0, const float* bcs, const float* diurnal_Q, const float* traj_bar,
+                  float* x0_bar, float* theta_bar, float* mpp_bar, size_t ncol);
+int cpz_solve_vjp_dev(cpz_model* m, const float* x0, const float* bcs, const float* diurnal_Q, const float* traj_bar,
+                      float* x0_bar, float* theta_bar, float* mpp_bar, size_t ncol);
+
 /* ---- S3: objective and gradient ------------------------------------------------------------- */
 /* replaces loss_NDE / loss_gradient_NDE + Zygote gradient (NDE_training.jl:290-333; loss.jl:1-42) and
  * nde_loss (free_convection/src/training.jl:55-62).
