@@ -44,6 +44,9 @@ int loss_grad_fc1(cpz_model* m, const float* x0, const float* bcs, const float* 
 int launch_closure(cpz_model* m, const ClosureD& cd, const ClosureArgs& a);
 int launch_closure_uvt(cpz_model* m, const ClosureUvtD& cd, const ClosureUvtArgs& a);
 int launch_closure_uvt_tc(cpz_model* m, const ClosureUvtD& cd, const ClosureUvtArgs& a);  // tcgen05 flavour (cpz_k_tc.cu); 1 = not eligible
+// pullback of the u/v/T closure step on the adjoint plan (cpz_k_closure_uvt_vjp.cu): persistent grid, one gradient slab per CTA
+struct ClosureUvtVjpArgs;  // cpz_closure_uvt_vjp.cuh
+int launch_closure_uvt_vjp(cpz_model* m, const ClosureUvtD& cd, const ClosureUvtVjpArgs& a, int grid);
 int launch_reduce_slabs(cpz_model* m, const float* part, int n_slabs, int P, float* out);
 int launch_pack_loss(cpz_model* m, const float* lpart, int n_slabs, int stride, float ncol, float* pack_tail);
 int launch_finalize_loss(cpz_model* m, const float* pack_tail, const float* w6, float inv_prof, float inv_grad, float* loss_out);

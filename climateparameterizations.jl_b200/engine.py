@@ -20,7 +20,8 @@ EXPORTS = [
     "cpz_model_n_params", "cpz_model_n_saved", "cpz_model_describe", "cpz_set_theta", "cpz_get_theta", "cpz_model_set_time", "cpz_rhs",
     "cpz_rhs_dev", "cpz_rhs_vjp", "cpz_rhs_vjp_dev", "cpz_predict_flux", "cpz_predict_flux_dev", "cpz_solve", "cpz_solve_dev", "cpz_solve_vjp", "cpz_solve_vjp_dev", "cpz_loss_grad", "cpz_loss_grad_dev", "cpz_train_step",
     "cpz_train_step_dev", "cpz_set_mpp_params", "cpz_get_mpp_params", "cpz_loss_grad_mpp", "cpz_loss_grad_mpp_dev", "cpz_adam_get_state", "cpz_adam_set_state", "cpz_closure_step", "cpz_closure_step_dev",
-    "cpz_sizeof_closure_uvt_desc", "cpz_closure_step_uvt", "cpz_closure_step_uvt_dev",
+    "cpz_sizeof_closure_uvt_desc", "cpz_closure_step_uvt", "cpz_closure_step_uvt_dev", "cpz_closure_step_uvt_vjp",
+    "cpz_closure_step_uvt_vjp_dev",
 ]
 
 ALLREDUCE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p)
@@ -88,6 +89,8 @@ def lib() -> C.CDLL:
         getattr(L, name).argtypes = [vp, C.POINTER(CClosureDesc), vp, vp, vp, vp]
     for name in ("cpz_closure_step_uvt", "cpz_closure_step_uvt_dev"):
         getattr(L, name).argtypes = [vp, C.POINTER(CClosureUvtDesc), vp, vp, vp, vp, vp]
+    for name in ("cpz_closure_step_uvt_vjp", "cpz_closure_step_uvt_vjp_dev"):
+        getattr(L, name).argtypes = [vp, C.POINTER(CClosureUvtDesc), vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     for name in EXPORTS:
         if name not in ("cpz_last_error", "cpz_sizeof_model_desc", "cpz_sizeof_closure_desc", "cpz_sizeof_closure_uvt_desc"):
             getattr(L, name).restype = C.c_int
@@ -386,6 +389,24 @@ class Model:
         _check(lib().cpz_closure_step_uvt(self._h, C.byref(c), _ptr(u), _ptr(v), _ptr(T), _ptr(dzf), _ptr(out)))
         return dzf, out
 
+    def closure_step_uvt_vjp(self, cdesc: ClosureUvtDesc, u, v, T, dz_flux_bar=None, uvT_bar=None, want_uvT: bool = True,
+                             want_theta: bool = True, want_mpp: bool = False):
+        """Pullback of closure_step_uvt() at (u, v, T) for the cotangents dz_flux_bar and uvT_bar [3,Nz,Ny,Nx] (None = zero) —
+        cpz_closure_step_uvt_vjp. Returns (uvT_bar_in [3,Nz,Ny,Nx] = u_bar, v_bar, T_bar; theta_bar [P]; mpp_bar [5] wrt
+        (nu0, nu_m, dRi, Ric, Pr)); an output that is not wanted is None."""
+        shp = (cdesc.Nz, cdesc.Ny, cdesc.Nx)
+        u, v, T = _np(u, shp), _np(v, shp), _np(T, shp)
+        fb = None if dz_flux_bar is None else _np(dz_flux_bar, (3,) + shp)
+        ob = None if uvT_bar is None else _np(uvT_bar, (3,) + shp)
+        xb = np.empty((3,) + shp, dtype=np.float32) if want_uvT else None
+        tb = np.empty(self.P, dtype=np.float32) if want_theta else None
+        pb = np.empty(5, dtype=np.float32) if want_mpp else None
+        c = cdesc.to_c()
+        q = (lambda i: None) if xb is None else (lambda i: xb[i])
+        _check(lib().cpz_closure_step_uvt_vjp(self._h, C.byref(c), _ptr(u), _ptr(v), _ptr(T), _ptr(fb), _ptr(ob), _ptr(q(0)),
+                                              _ptr(q(1)), _ptr(q(2)), _ptr(tb), _ptr(pb)))
+        return xb, tb, pb
+
     # -- device-pointer flavour (torch CUDA tensors or raw addresses; enqueued on the context's stream, no sync)
     def rhs_dev(self, x, bcs, out, t: float = 0.0, Q=None, ncol: Optional[int] = None) -> None:
         ncol = ncol if ncol is not None else x.shape[0]
@@ -431,6 +452,14 @@ class Model:
     def closure_step_uvt_dev(self, cdesc: ClosureUvtDesc, u, v, T, dz_flux, uvT_out) -> None:
         c = cdesc.to_c()
         _check(lib().cpz_closure_step_uvt_dev(self._h, C.byref(c), _ptr(u), _ptr(v), _ptr(T), _ptr(dz_flux), _ptr(uvT_out)))
+
+    def closure_step_uvt_vjp_dev(self, cdesc: ClosureUvtDesc, u, v, T, dz_flux_bar=None, uvT_bar=None, u_bar=None, v_bar=None,
+                                 T_bar=None, theta_bar=None, mpp_bar=None) -> None:
+        """cpz_closure_step_uvt_vjp_dev: the outputs given (u_bar, v_bar, T_bar [Nz,Ny,Nx], theta_bar [P], mpp_bar [5]) are
+        overwritten."""
+        c = cdesc.to_c()
+        _check(lib().cpz_closure_step_uvt_vjp_dev(self._h, C.byref(c), _ptr(u), _ptr(v), _ptr(T), _ptr(dz_flux_bar), _ptr(uvT_bar),
+                                                  _ptr(u_bar), _ptr(v_bar), _ptr(T_bar), _ptr(theta_bar), _ptr(mpp_bar)))
 
     def close(self) -> None:
         if self._h:

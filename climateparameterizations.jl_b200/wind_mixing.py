@@ -450,3 +450,55 @@ def oceananigans_modified_pacanowski_philander_nn(model: engine.Model, cdesc, u,
         if (it + 1) % output_every == 0:
             frames.append((u.copy(), v.copy(), T.copy()))
     return frames
+
+
+def closure_step_uvt_autograd(model: engine.Model, cdesc, theta, u, v, T):
+    """One embedded closure step (cpz_closure_step_uvt_dev) as a torch autograd node whose backward is
+    cpz_closure_step_uvt_vjp_dev: (dz_flux [3,Nz,Ny,Nx], uvT' [3,Nz,Ny,Nx]) of CUDA float32 fields [Nz,Ny,Nx] on the model's
+    device. `theta` ([P] tensor) is copied into the model first and receives theta_bar; u, v, T receive their cotangents. A host
+    model written in torch can chain through several closure steps and train the nets "a posteriori" on the discretisation
+    they are deployed in."""
+    global _CLOSURE_STEP_UVT
+    if _CLOSURE_STEP_UVT is None:  # built on first use: importing this module does not import torch
+        _CLOSURE_STEP_UVT = _closure_autograd_function()
+    return _CLOSURE_STEP_UVT.apply(model, cdesc, theta, u, v, T)
+
+
+_CLOSURE_STEP_UVT = None
+
+
+def _closure_autograd_function():
+    import torch
+
+    class ClosureStepUvt(torch.autograd.Function):
+        @staticmethod
+        def forward(fctx, model, cdesc, theta, u, v, T):
+            model.set_theta(theta.detach().float().cpu().numpy())
+            u, v, T = (a.detach().float().contiguous() for a in (u, v, T))
+            dzf = torch.empty((3,) + tuple(u.shape), device=u.device)
+            out = torch.empty_like(dzf)
+            torch.cuda.synchronize(u.device)
+            model.closure_step_uvt_dev(cdesc, u, v, T, dzf, out)
+            model.ctx.synchronize()
+            fctx.model, fctx.cdesc, fctx.theta_meta = model, cdesc, (theta.dtype, theta.device)
+            fctx.save_for_backward(u, v, T)
+            return dzf, out
+
+        @staticmethod
+        def backward(fctx, dzf_bar, out_bar):
+            u, v, T = fctx.saved_tensors
+            m = fctx.model
+            fb = None if dzf_bar is None else dzf_bar.float().contiguous()
+            ob = None if out_bar is None else out_bar.float().contiguous()
+            if fb is None and ob is None:
+                return None, None, None, None, None, None
+            xb = torch.empty((3,) + tuple(u.shape), device=u.device)
+            tb = torch.empty(m.P, device=u.device)
+            torch.cuda.synchronize(u.device)
+            m.closure_step_uvt_vjp_dev(fctx.cdesc, u, v, T, fb, ob, xb[0], xb[1], xb[2], tb)
+            m.ctx.synchronize()
+            dtype, device = fctx.theta_meta
+            return None, None, tb.to(dtype=dtype, device=device), xb[0], xb[1], xb[2]
+
+    return ClosureStepUvt
+

@@ -317,6 +317,28 @@ int cpz_closure_step_uvt(cpz_model* m, const cpz_closure_uvt_desc* c, const floa
 int cpz_closure_step_uvt_dev(cpz_model* m, const cpz_closure_uvt_desc* c, const float* u, const float* v, const float* T,
                              float* dz_flux_out, float* uvT_out);
 
+/* pullback of cpz_closure_step_uvt at (u, v, T) on the same model, theta and mPP parameters, for the cotangents dz_flux_bar of
+ * dz_flux_out and uvT_bar of uvT_out (both [3][Nz][Ny][Nx]; either may be NULL = zero, not both). Lets a host that
+ * differentiates its own ocean or column model (Zygote / Enzyme over a Julia host, torch autograd over a Python one) chain
+ * through the closure and train the nets, or tune the base closure, on the discretisation they are deployed in:
+ *   u_bar, v_bar, T_bar: [Nz][Ny][Nx] cotangents of the incoming fields;
+ *   theta_bar: [P], summed over all columns, destructure order (NULL required when P = 0);
+ *   mpp_bar[5]: wrt p = (nu0, nu_m, dRi, Ric, Pr), unscaled, as cpz_loss_grad_mpp (refused with smooth_Ri).
+ * The step's outputs depend on the state through separate paths: dz_flux through the nets, (u', v', T') through the implicit
+ * mPP step of the incoming state (the forcing is applied by the host), so theta_bar comes from dz_flux_bar alone and mpp_bar
+ * from uvT_bar alone. uw_top, vw_top and wT_top are additive constants and drop out. T'[bottom] = T[bottom] and nu = 0 on
+ * the two boundary faces are differentiated as the forward states them. At relu kinks and at the convective-adjustment
+ * switch the derivative is that of the branch the forward evaluated. Outputs are overwritten, not accumulated, and each may
+ * be NULL (not all). The sums over columns run in a fixed order (bitwise reproducible); the allreduce hook is not called
+ * and there is no non-finite reporting. The argument checks are cpz_closure_step_uvt's; a model without the adjoint plan
+ * (e.g. the 400-wide nets) is refused with the planner's reason. */
+int cpz_closure_step_uvt_vjp(cpz_model* m, const cpz_closure_uvt_desc* c, const float* u, const float* v, const float* T,
+                             const float* dz_flux_bar, const float* uvT_bar, float* u_bar, float* v_bar, float* T_bar,
+                             float* theta_bar, float* mpp_bar);
+int cpz_closure_step_uvt_vjp_dev(cpz_model* m, const cpz_closure_uvt_desc* c, const float* u, const float* v, const float* T,
+                                 const float* dz_flux_bar, const float* uvT_bar, float* u_bar, float* v_bar, float* T_bar,
+                                 float* theta_bar, float* mpp_bar);
+
 #ifdef __cplusplus
 }
 #endif
