@@ -10,6 +10,7 @@
 
 #include "cpz_launch.h"
 #include "cpz_closure_uvt_vjp.cuh"
+#include "cpz_closure_vjp.cuh"
 
 namespace cpz {
 
@@ -313,6 +314,12 @@ int cpz_model_describe(const cpz_model* m, char* buf, size_t buf_len) {
   }
   if (m->has_bwd && m->desc.n_fields == 3 && m->desc.n_nets == 3) {
     snprintf(line, sizeof(line), "u/v/T closure-step pullback (cpz_closure_step_uvt_vjp): closure_uvt_vjp_kernel, fp32-simt, 32-column tiles "
+             "(32 consecutive x-columns) on the adjoint plan, weights %s, persistent grid of min(tiles, %d) CTAs with one gradient slab each\n",
+             m->bwd.M.w_in_smem ? "in shared memory" : "streamed from global memory", m->ctx->sm_count);
+    s += line;
+  }
+  if (m->has_bwd && m->desc.n_fields == 1 && m->desc.n_nets == 1) {
+    snprintf(line, sizeof(line), "gyre closure-step pullback (cpz_closure_step_vjp): closure_vjp_kernel, fp32-simt, 32-column tiles "
              "(32 consecutive x-columns) on the adjoint plan, weights %s, persistent grid of min(tiles, %d) CTAs with one gradient slab each\n",
              m->bwd.M.w_in_smem ? "in shared memory" : "streamed from global memory", m->ctx->sm_count);
     s += line;

@@ -47,6 +47,9 @@ int launch_closure_uvt_tc(cpz_model* m, const ClosureUvtD& cd, const ClosureUvtA
 // pullback of the u/v/T closure step on the adjoint plan (cpz_k_closure_uvt_vjp.cu): persistent grid, one gradient slab per CTA
 struct ClosureUvtVjpArgs;  // cpz_closure_uvt_vjp.cuh
 int launch_closure_uvt_vjp(cpz_model* m, const ClosureUvtD& cd, const ClosureUvtVjpArgs& a, int grid);
+// pullback of the gyre closure step on the adjoint plan (cpz_k_closure_vjp.cu): persistent grid, one gradient slab per CTA
+struct ClosureVjpArgs;  // cpz_closure_vjp.cuh
+int launch_closure_vjp(cpz_model* m, const ClosureD& cd, const ClosureVjpArgs& a, int grid);
 int launch_reduce_slabs(cpz_model* m, const float* part, int n_slabs, int P, float* out);
 int launch_pack_loss(cpz_model* m, const float* lpart, int n_slabs, int stride, float ncol, float* pack_tail);
 int launch_finalize_loss(cpz_model* m, const float* pack_tail, const float* w6, float inv_prof, float inv_grad, float* loss_out);

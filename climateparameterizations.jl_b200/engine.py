@@ -21,7 +21,7 @@ EXPORTS = [
     "cpz_rhs_dev", "cpz_rhs_vjp", "cpz_rhs_vjp_dev", "cpz_predict_flux", "cpz_predict_flux_dev", "cpz_solve", "cpz_solve_dev", "cpz_solve_vjp", "cpz_solve_vjp_dev", "cpz_loss_grad", "cpz_loss_grad_dev", "cpz_train_step",
     "cpz_train_step_dev", "cpz_set_mpp_params", "cpz_get_mpp_params", "cpz_loss_grad_mpp", "cpz_loss_grad_mpp_dev", "cpz_adam_get_state", "cpz_adam_set_state", "cpz_closure_step", "cpz_closure_step_dev",
     "cpz_sizeof_closure_uvt_desc", "cpz_closure_step_uvt", "cpz_closure_step_uvt_dev", "cpz_closure_step_uvt_vjp",
-    "cpz_closure_step_uvt_vjp_dev",
+    "cpz_closure_step_uvt_vjp_dev", "cpz_closure_step_vjp", "cpz_closure_step_vjp_dev",
 ]
 
 ALLREDUCE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p)
@@ -87,6 +87,8 @@ def lib() -> C.CDLL:
     L.cpz_adam_set_state.argtypes = [vp, vp, vp, vp, sz]
     for name in ("cpz_closure_step", "cpz_closure_step_dev"):
         getattr(L, name).argtypes = [vp, C.POINTER(CClosureDesc), vp, vp, vp, vp]
+    for name in ("cpz_closure_step_vjp", "cpz_closure_step_vjp_dev"):
+        getattr(L, name).argtypes = [vp, C.POINTER(CClosureDesc), vp, vp, vp, vp, vp]
     for name in ("cpz_closure_step_uvt", "cpz_closure_step_uvt_dev"):
         getattr(L, name).argtypes = [vp, C.POINTER(CClosureUvtDesc), vp, vp, vp, vp, vp]
     for name in ("cpz_closure_step_uvt_vjp", "cpz_closure_step_uvt_vjp_dev"):
@@ -379,6 +381,20 @@ class Model:
         _check(lib().cpz_closure_step(self._h, C.byref(c), _ptr(T), _ptr(y), _ptr(forcing), _ptr(T_out)))
         return forcing, T_out
 
+    def closure_step_vjp(self, cdesc: ClosureDesc, T, forcing_bar=None, T_out_bar=None, want_T: bool = True,
+                         want_theta: bool = True):
+        """Pullback of closure_step() at T for the cotangents forcing_bar and T_out_bar [Nz,Ny,Nx] (None = zero) —
+        cpz_closure_step_vjp. Returns (T_bar [Nz,Ny,Nx], theta_bar [P]); an output that is not wanted is None."""
+        shp = (cdesc.Nz, cdesc.Ny, cdesc.Nx)
+        T = _np(T, shp)
+        fb = None if forcing_bar is None else _np(forcing_bar, shp)
+        ob = None if T_out_bar is None else _np(T_out_bar, shp)
+        xb = np.empty(shp, dtype=np.float32) if want_T else None
+        tb = np.empty(self.P, dtype=np.float32) if want_theta else None
+        c = cdesc.to_c()
+        _check(lib().cpz_closure_step_vjp(self._h, C.byref(c), _ptr(T), _ptr(fb), _ptr(ob), _ptr(xb), _ptr(tb)))
+        return xb, tb
+
     def closure_step_uvt(self, cdesc: ClosureUvtDesc, u, v, T):
         """One host-model step of the embedded u/v/T NDE: (dz_flux [3,Nz,Ny,Nx], uvT' [3,Nz,Ny,Nx]); fields are [Nz,Ny,Nx]."""
         shp = (cdesc.Nz, cdesc.Ny, cdesc.Nx)
@@ -448,6 +464,12 @@ class Model:
     def closure_step_dev(self, cdesc: ClosureDesc, T, y, forcing, T_out) -> None:
         c = cdesc.to_c()
         _check(lib().cpz_closure_step_dev(self._h, C.byref(c), _ptr(T), _ptr(y), _ptr(forcing), _ptr(T_out)))
+
+    def closure_step_vjp_dev(self, cdesc: ClosureDesc, T, forcing_bar=None, T_out_bar=None, T_bar=None, theta_bar=None) -> None:
+        """cpz_closure_step_vjp_dev: the outputs given (T_bar [Nz,Ny,Nx], theta_bar [P]) are overwritten."""
+        c = cdesc.to_c()
+        _check(lib().cpz_closure_step_vjp_dev(self._h, C.byref(c), _ptr(T), _ptr(forcing_bar), _ptr(T_out_bar), _ptr(T_bar),
+                                              _ptr(theta_bar)))
 
     def closure_step_uvt_dev(self, cdesc: ClosureUvtDesc, u, v, T, dz_flux, uvT_out) -> None:
         c = cdesc.to_c()

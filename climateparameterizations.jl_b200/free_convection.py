@@ -200,3 +200,55 @@ def train_neural_differential_equation(NN: Chain, NDEType, algorithm, datasets: 
         m.close()
         if own:
             ctx.close()
+
+
+def closure_step_autograd(model: engine.Model, cdesc, theta, T, y):
+    """One gyre closure step (cpz_closure_step_dev) as a torch autograd node whose backward is cpz_closure_step_vjp_dev:
+    (forcing [Nz,Ny,Nx], T' [Nz,Ny,Nx]) of a CUDA float32 field T [Nz,Ny,Nx] and y [Ny] on the model's device. `theta` ([P]
+    tensor) is copied into the model first and receives theta_bar; T receives T_bar, y no cotangent (it enters the forcing
+    additively). A host model written in torch can chain through several closure steps and train the T-only net
+    "a posteriori" on the discretisation it is deployed in."""
+    global _CLOSURE_STEP
+    if _CLOSURE_STEP is None:  # built on first use: importing this module does not import torch
+        _CLOSURE_STEP = _closure_autograd_function()
+    return _CLOSURE_STEP.apply(model, cdesc, theta, T, y)
+
+
+_CLOSURE_STEP = None
+
+
+def _closure_autograd_function():
+    import torch
+
+    class ClosureStep(torch.autograd.Function):
+        @staticmethod
+        def forward(fctx, model, cdesc, theta, T, y):
+            model.set_theta(theta.detach().float().cpu().numpy())
+            T = T.detach().float().contiguous()
+            y = y.detach().float().contiguous()
+            forcing = torch.empty_like(T)
+            T_out = torch.empty_like(T)
+            torch.cuda.synchronize(T.device)
+            model.closure_step_dev(cdesc, T, y, forcing, T_out)
+            model.ctx.synchronize()
+            fctx.model, fctx.cdesc, fctx.theta_meta = model, cdesc, (theta.dtype, theta.device)
+            fctx.save_for_backward(T)
+            return forcing, T_out
+
+        @staticmethod
+        def backward(fctx, forcing_bar, T_out_bar):
+            (T,) = fctx.saved_tensors
+            m = fctx.model
+            fb = None if forcing_bar is None else forcing_bar.float().contiguous()
+            ob = None if T_out_bar is None else T_out_bar.float().contiguous()
+            if fb is None and ob is None:
+                return None, None, None, None, None
+            Tb = torch.empty_like(T)
+            tb = torch.empty(m.P, device=T.device)
+            torch.cuda.synchronize(T.device)
+            m.closure_step_vjp_dev(fctx.cdesc, T, fb, ob, Tb, tb)
+            m.ctx.synchronize()
+            dtype, device = fctx.theta_meta
+            return None, None, tb.to(dtype=dtype, device=device), Tb, None
+
+    return ClosureStep

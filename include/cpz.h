@@ -293,6 +293,24 @@ int cpz_closure_step(cpz_model* m, const cpz_closure_desc* c, const float* T, co
 int cpz_closure_step_dev(cpz_model* m, const cpz_closure_desc* c, const float* T, const float* y, float* forcing_out,
                          float* T_out);
 
+/* pullback of cpz_closure_step at T on the same model and theta, for the cotangents forcing_bar of forcing_out and T_out_bar
+ * of T_out (both [Nz][Ny][Nx]; either may be NULL = zero, not both). Lets a host that differentiates its gyre model (Zygote /
+ * Enzyme over a Julia host, torch autograd over a Python one) chain through the closure and train the T-only net on the
+ * discretisation it is deployed in:
+ *   T_bar: [Nz][Ny][Nx] cotangent of the incoming T;
+ *   theta_bar: [P], summed over all columns, destructure order.
+ * T' = A(T)^-1 T is the implicit convective adjustment; the forcing depends on T' through the net and the surface restoring
+ * flux, so theta_bar comes from forcing_bar alone (T_out_bar alone gives theta_bar = 0 exactly), and T_bar = A^-1 (T_out_bar
+ * + the forcing path's cotangent of T') with A symmetric. y, T_mid, dT and Ly are additive constants and drop out, so the
+ * pullback takes no y. At relu kinks and at the convective-adjustment switch the derivative is that of the branch the forward
+ * evaluated. Outputs are overwritten, not accumulated, and each may be NULL (not both). The sums over columns run in a fixed
+ * order (bitwise reproducible); the allreduce hook is not called and there is no non-finite reporting. The argument checks
+ * are cpz_closure_step's; a model without the adjoint plan is refused with the planner's reason. */
+int cpz_closure_step_vjp(cpz_model* m, const cpz_closure_desc* c, const float* T, const float* forcing_bar,
+                         const float* T_out_bar, float* T_bar, float* theta_bar);
+int cpz_closure_step_vjp_dev(cpz_model* m, const cpz_closure_desc* c, const float* T, const float* forcing_bar,
+                             const float* T_out_bar, float* T_bar, float* theta_bar);
+
 /* ---- S7b: per-step closure of the u/v/T NDE inside a host ocean model (SURVEY 8f-2) ---------- */
 /* replaces the Simulation callback progress_neural_network (wind_mixing/src/NDE_oceananigans.jl:380-405): the NN forcing
  * chains NN_uw_forcing / NN_vw_forcing / NN_wT_forcing on the incoming state (:288-344; dz of [0; unscaled NN - shift;
