@@ -450,6 +450,47 @@ __device__ __forceinline__ int last_layer_of(const ModelD& M) {
   return L;
 }
 
+// MLP forward keeping z and a for mlp_backward_layer. The last layer's outputs are not needed (everything downstream of
+// the nets is affine in them), so its phases are skipped. Each phase ends with a block barrier.
+template <int CT, int NT, bool WS>
+__device__ __forceinline__ void mlp_forward_keep(const ModelD& M, int Lmax, const PhaseCache& pc, const float* in, float* arena,
+                                                 float* zarena, const float* wsm, const float* theta) {
+  for (int p = 0; p < M.n_phase; ++p) {
+    if (M.gemm[M.phase[p].g0].layer == Lmax && M.gemm[M.phase[p].g1 - 1].layer == Lmax) continue;
+    run_phase_cached<CT, NT, WS, true>(M, p, pc, in, arena, zarena, wsm, theta);
+    __syncthreads();
+  }
+}
+
+// Reverse of the MLP, last layer first, from the NN-output cotangents in zarena: weight gradients into gpart, the input
+// cotangent added to xb. Each layer ends with a block barrier.
+template <int CT, int NT, bool WS>
+__device__ __forceinline__ void mlp_backward(const ModelD& M, int Lmax, const float* in, const float* arena, float* zarena,
+                                             float* xb, const float* wsm, const float* theta, float* gpart) {
+  for (int l = Lmax; l >= 0; --l) {
+    mlp_backward_layer<WS, CT, NT>(M, l, in, arena, zarena, xb, wsm, theta, gpart);
+    __syncthreads();
+  }
+}
+
+// Block reduction (fixed order) of the five FP64 mPP-parameter sums into this CTA's lpart row at LP/2 .. LP/2+4.
+// red: NT/32 floats of shared scratch.
+template <int NT>
+__device__ __forceinline__ void store_pgrad_sums(const double (&pgs)[5], float* red, float* lpart) {
+  for (int q = 0; q < 5; ++q) {
+    double vd = pgs[q];
+    for (int o = 16; o > 0; o >>= 1) vd += __shfl_xor_sync(0xffffffffu, vd, o);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = (float)vd;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      float s = 0.f;
+      for (int wdx = 0; wdx < NT / 32; ++wdx) s += red[wdx];
+      lpart[(size_t)blockIdx.x * LP + LP / 2 + q] = s;
+    }
+    __syncthreads();
+  }
+}
+
 // loss terms at one saved frame: accumulates the 6 squared-error sums and adds d(loss)/dx to xbar.
 // x: state tile, tg: target tile (same layout). Invalid columns (c >= nvalid) contribute nothing.
 template <int CT, int NT>
@@ -801,12 +842,7 @@ __device__ __forceinline__ void adjoint_body(const ModelD& M, const ModelD& Mp, 
           __syncthreads();
           CPZ_APROF_ADD(1, pb0);
           const long long pb1 = CPZ_APROF_T();
-          // MLP forward keeping z and a (the last layer's outputs are not needed: F is linear in them)
-          for (int p = 0; p < M.n_phase; ++p) {
-            if (M.gemm[M.phase[p].g0].layer == Lmax && M.gemm[M.phase[p].g1 - 1].layer == Lmax) continue;
-            run_phase_cached<CT, NT, WS, true>(M, p, pc, in, arena, zarena, wsm, a.theta);
-            __syncthreads();
-          }
+          mlp_forward_keep<CT, NT, WS>(M, Lmax, pc, in, arena, zarena, wsm, a.theta);
           CPZ_APROF_ADD(2, pb1);
           const long long pb2 = CPZ_APROF_T();
           faces_vjp<CT, NT>(M, in, xb, zarena, gflux, a.want_pgrad ? pgs : nullptr);

@@ -1,4 +1,5 @@
-// Launcher of adjoint_kernel<CT,NT,WS,COT> shared by the 32-column (cpz_k_adjoint.cu) and small-tile (cpz_k_small.cu) translation units.
+// Launcher of adjoint_kernel<CT,NT,WS,COT> shared by the 32-column (cpz_k_adjoint.cu) and small-tile (cpz_k_small.cu) translation
+// units, and of the single-evaluation pullbacks (cpz_k_rhs_vjp.cu, cpz_k_closure_vjp.cu, cpz_k_closure_uvt_vjp.cu).
 #pragma once
 #include <cstdio>
 #include <cstdlib>
@@ -39,5 +40,26 @@ static int launch_adjoint_t(cpz_model* m, const Plan& plan, const AdjArgs& a, in
   return CPZ_OK;
 }
 
+// Launcher of a single-evaluation pullback on the adjoint plan (VJP_NT threads, VJP_CT-column tiles, the caller has checked
+// has_bwd): kern_ws / kern_wg are its instantiations with the weights in shared memory / streamed from global memory, taking
+// the plan's ModelD and then `args`. scratch_rows: rows of the activation arena and zarena (adjacent in adjoint_smem_layout)
+// that the kernel borrows as scratch outside the MLP.
+template <class... Args>
+static int launch_vjp_t(cpz_model* m, void (*kern_ws)(ModelD, Args...), void (*kern_wg)(ModelD, Args...), const char* name,
+                        int scratch_rows, int grid, const Args&... args) {
+  const ModelD& M = m->bwd.M;
+  if (M.arena_floats + M.flux_off < scratch_rows)
+    return fail(CPZ_ERR_INVALID, "%s: the adjoint plan's activation arena (%d rows) is smaller than the %d rows of the kernel's scratch",
+                name, M.arena_floats + M.flux_off, scratch_rows);
+  const AdjSmem L = adjoint_smem_layout(M, VJP_CT);  // the adjoint plan was built to fit this layout
+  const size_t smem = (size_t)L.total_floats * sizeof(float);
+  if (smem > m->ctx->smem_optin) return fail(CPZ_ERR_INVALID, "%s kernel needs %zu B shared memory, device allows %zu", name, smem, m->ctx->smem_optin);
+  auto kern = M.w_in_smem ? kern_ws : kern_wg;
+  CPZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<grid, VJP_NT, smem, m->ctx->stream>>>(M, args...);
+  CPZ_CUDA(cudaGetLastError());
+  m->ctx->launches++;
+  return CPZ_OK;
+}
 
 }  // namespace cpz

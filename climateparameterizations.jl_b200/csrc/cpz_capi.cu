@@ -47,6 +47,56 @@ static void release(DevBuf& b) {
   b.p = nullptr; b.cap = 0;
 }
 
+// Grid and reduction buffers of the single-evaluation pullbacks (cpz_rhs_vjp, cpz_closure_step_vjp,
+// cpz_closure_step_uvt_vjp): a persistent grid of min(tiles, SMs) CTAs over VJP_CT-column tiles, each CTA with one
+// weight-gradient slab in b_part and one LP row after the slabs. b_red is touched only when mpp_bar is wanted: host flavours
+// stage theta_bar in b_red[0, P) and grow b_red to P + 16 beforehand, so the ensure here never reallocates an output they
+// passed in.
+struct SlabPullback {
+  float* theta_bar;  // [P] output, or null
+  float* mpp_bar;    // [5] output, or null
+  size_t ncol;
+  int n_tiles, grid;
+  float* gpart;  // [grid][M.slab] weight-gradient slabs, zeroed when theta_bar is wanted
+  float* lpart;  // [grid][LP], zeroed when mpp_bar is wanted: the five mPP-parameter sums at LP/2 .. LP/2+4
+};
+
+static int begin_slab_pullback(cpz_model* m, size_t ncol, float* theta_bar, float* mpp_bar, SlabPullback& sp) {
+  cudaStream_t st = m->ctx->stream;
+  sp.theta_bar = theta_bar; sp.mpp_bar = mpp_bar; sp.ncol = ncol;
+  sp.n_tiles = (int)((ncol + VJP_CT - 1) / VJP_CT);
+  sp.grid = std::min(sp.n_tiles, m->ctx->sm_count);
+  const size_t slab = (size_t)m->bwd.M.slab;
+  int rc;
+  if ((rc = ensure(m->b_part, (size_t)sp.grid * (slab + LP)))) return rc;
+  if (mpp_bar && (rc = ensure(m->b_red, m->P + 16))) return rc;
+  sp.gpart = m->b_part.p;
+  sp.lpart = m->b_part.p + (size_t)sp.grid * slab;
+  if (theta_bar) CPZ_CUDA(cudaMemsetAsync(sp.gpart, 0, (size_t)sp.grid * slab * sizeof(float), st));
+  if (mpp_bar) CPZ_CUDA(cudaMemsetAsync(sp.lpart, 0, (size_t)sp.grid * LP * sizeof(float), st));
+  return CPZ_OK;
+}
+
+// theta_bar = the sum of the slabs; mpp_bar = the five mPP-parameter sums of the LP rows
+static int finish_slab_pullback(cpz_model* m, const SlabPullback& sp) {
+  const int P = (int)m->P;
+  int rc;
+  if (sp.theta_bar && (rc = launch_reduce_slabs(m, sp.gpart, sp.grid, P, sp.theta_bar))) return rc;
+  if (sp.mpp_bar) {
+    if ((rc = launch_pack_loss(m, sp.lpart, sp.grid, LP, (float)sp.ncol, m->b_red.p + P))) return rc;
+    CPZ_CUDA(cudaMemcpyAsync(sp.mpp_bar, m->b_red.p + P + 8, 5 * sizeof(float), cudaMemcpyDeviceToDevice, m->ctx->stream));
+  }
+  return CPZ_OK;
+}
+
+// The mPP-parameter gradient (cpz_loss_grad_mpp, and mpp_bar of the pullbacks that run the model's own RHS)
+static int check_mpp_grad(const cpz_model* m) {
+  if (m->desc.n_fields != 3) return fail(CPZ_ERR_INVALID, "mPP-parameter gradient needs the u/v/T model");
+  if (!((m->desc.flags & CPZ_FLAG_MPP) || m->desc.variant == CPZ_RHS_INFER)) return fail(CPZ_ERR_INVALID, "mPP-parameter gradient needs CPZ_FLAG_MPP");
+  if (m->desc.flags & CPZ_FLAG_SMOOTH_RI) return fail(CPZ_ERR_INVALID, "mPP-parameter gradient is not available with smooth_Ri");
+  return CPZ_OK;
+}
+
 static int n_saved_of(const TimeD& tm) { return tm.save_stride <= 0 ? 1 : tm.n_steps / tm.save_stride + 1; }
 // checkpoints: step 0, every ckpt_stride-th step, and the final step (once)
 static int n_ckpt_of(const TimeD& tm) {
@@ -306,24 +356,17 @@ int cpz_model_describe(const cpz_model* m, char* buf, size_t buf_len) {
   dump("forward", m->fwd, solve_other_smem(m->desc, m->CT, m->tab.n_stages));
   if (m->has_bwd) dump("adjoint", m->bwd, adjoint_other_smem(m->desc.n_fields * m->desc.Nz, m->desc.n_fields == 3 ? 6 : 2, m->CT));
   else s += "adjoint plan: unavailable (" + m->bwd_err + ")\n";
-  if (m->has_bwd) {
-    snprintf(line, sizeof(line), "rhs pullback (cpz_rhs_vjp): rhs_vjp_kernel, fp32-simt, 32-column tiles on the adjoint plan, weights %s, "
-             "persistent grid of min(tiles, %d) CTAs with one gradient slab each\n",
+  auto pullback = [&](const char* what, const char* kernel, bool closure) {  // the single-evaluation pullbacks (launch_vjp_t)
+    snprintf(line, sizeof(line), "%s: %s, fp32-simt, 32-column tiles%s on the adjoint plan, weights %s, persistent grid of min(tiles, %d) "
+             "CTAs with one gradient slab each\n", what, kernel, closure ? " (32 consecutive x-columns)" : "",
              m->bwd.M.w_in_smem ? "in shared memory" : "streamed from global memory", m->ctx->sm_count);
     s += line;
-  }
-  if (m->has_bwd && m->desc.n_fields == 3 && m->desc.n_nets == 3) {
-    snprintf(line, sizeof(line), "u/v/T closure-step pullback (cpz_closure_step_uvt_vjp): closure_uvt_vjp_kernel, fp32-simt, 32-column tiles "
-             "(32 consecutive x-columns) on the adjoint plan, weights %s, persistent grid of min(tiles, %d) CTAs with one gradient slab each\n",
-             m->bwd.M.w_in_smem ? "in shared memory" : "streamed from global memory", m->ctx->sm_count);
-    s += line;
-  }
-  if (m->has_bwd && m->desc.n_fields == 1 && m->desc.n_nets == 1) {
-    snprintf(line, sizeof(line), "gyre closure-step pullback (cpz_closure_step_vjp): closure_vjp_kernel, fp32-simt, 32-column tiles "
-             "(32 consecutive x-columns) on the adjoint plan, weights %s, persistent grid of min(tiles, %d) CTAs with one gradient slab each\n",
-             m->bwd.M.w_in_smem ? "in shared memory" : "streamed from global memory", m->ctx->sm_count);
-    s += line;
-  }
+  };
+  if (m->has_bwd) pullback("rhs pullback (cpz_rhs_vjp)", "rhs_vjp_kernel", false);
+  if (m->has_bwd && m->desc.n_fields == 3 && m->desc.n_nets == 3)
+    pullback("u/v/T closure-step pullback (cpz_closure_step_uvt_vjp)", "closure_uvt_vjp_kernel", true);
+  if (m->has_bwd && m->desc.n_fields == 1 && m->desc.n_nets == 1)
+    pullback("gyre closure-step pullback (cpz_closure_step_vjp)", "closure_vjp_kernel", true);
   s += "solve pullback (cpz_solve_vjp): the cpz_loss_grad kernels above in cotangent mode (the trajectory cotangent replaces the "
        "loss terms at the saved frames; x0 cotangent stored at the end of the reverse sweep)\n";
   if (m->has_small[0]) {
@@ -435,34 +478,17 @@ int cpz_rhs_vjp_dev(cpz_model* m, const float* x, const float* bcs, const float*
   if (!x || !bcs || !dxdt_bar) return fail(CPZ_ERR_INVALID, "null array");
   if ((m->desc.flags & CPZ_FLAG_DIURNAL) && !diurnal_Q) return fail(CPZ_ERR_INVALID, "diurnal model needs diurnal_Q");
   if (theta_bar && m->P == 0) return fail(CPZ_ERR_INVALID, "rhs_vjp: theta_bar requested but the model has no parameters");
-  if (mpp_bar) {  // the checks of cpz_loss_grad_mpp
-    if (m->desc.n_fields != 3) return fail(CPZ_ERR_INVALID, "mPP-parameter gradient needs the u/v/T model");
-    if (!((m->desc.flags & CPZ_FLAG_MPP) || m->desc.variant == CPZ_RHS_INFER)) return fail(CPZ_ERR_INVALID, "mPP-parameter gradient needs CPZ_FLAG_MPP");
-    if (m->desc.flags & CPZ_FLAG_SMOOTH_RI) return fail(CPZ_ERR_INVALID, "mPP-parameter gradient is not available with smooth_Ri");
-  }
+  if (mpp_bar && (rc = check_mpp_grad(m))) return rc;
   if (!m->has_bwd) return fail(CPZ_ERR_INVALID, "adjoint plan unavailable: %s", m->bwd_err.c_str());
   if (ncol > (size_t)INT32_MAX / 512) return fail(CPZ_ERR_INVALID, "ncol too large");
   if ((rc = bind_device(m->ctx))) return rc;
-  cudaStream_t st = m->ctx->stream;
-  const int P = (int)m->P;
-  const int n_tiles = (int)((ncol + m->CT - 1) / m->CT);
-  const int grid = std::min(n_tiles, m->ctx->sm_count);
-  const size_t slab = (size_t)m->bwd.M.slab;
-  if ((rc = ensure(m->b_part, (size_t)grid * (slab + LP)))) return rc;
-  if ((rc = ensure(m->b_red, (size_t)P + 16))) return rc;
-  float* lpart = m->b_part.p + (size_t)grid * slab;
-  if (theta_bar) CPZ_CUDA(cudaMemsetAsync(m->b_part.p, 0, (size_t)grid * slab * sizeof(float), st));
-  if (mpp_bar) CPZ_CUDA(cudaMemsetAsync(lpart, 0, (size_t)grid * LP * sizeof(float), st));
+  SlabPullback sp;
+  if ((rc = begin_slab_pullback(m, ncol, theta_bar, mpp_bar, sp))) return rc;
   VjpArgs a{};
-  a.theta = m->d_theta; a.x = x; a.ybar = dxdt_bar; a.xbar = x_bar; a.gpart = m->b_part.p; a.lpart = lpart;
-  a.want_mlp = (x_bar || theta_bar) && P > 0; a.want_pgrad = mpp_bar != nullptr; a.ncol = (int)ncol; a.n_tiles = n_tiles;
-  if ((rc = launch_rhs_vjp(m, a, grid))) return rc;
-  if (theta_bar && (rc = launch_reduce_slabs(m, m->b_part.p, grid, P, theta_bar))) return rc;
-  if (mpp_bar) {
-    if ((rc = launch_pack_loss(m, lpart, grid, LP, (float)ncol, m->b_red.p + P))) return rc;
-    CPZ_CUDA(cudaMemcpyAsync(mpp_bar, m->b_red.p + P + 8, 5 * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  }
-  return CPZ_OK;
+  a.theta = m->d_theta; a.x = x; a.ybar = dxdt_bar; a.xbar = x_bar; a.gpart = sp.gpart; a.lpart = sp.lpart;
+  a.want_mlp = (x_bar || theta_bar) && m->P > 0; a.want_pgrad = mpp_bar != nullptr; a.ncol = (int)ncol; a.n_tiles = sp.n_tiles;
+  if ((rc = launch_rhs_vjp(m, a, sp.grid))) return rc;
+  return finish_slab_pullback(m, sp);
 }
 
 int cpz_rhs_vjp(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, const float* dxdt_bar,

@@ -10,7 +10,7 @@
 //   nubar_f = -r (lambda_f - lambda_{f-1}) (y_f - y_{f-1})   (y: the solve's output, before the T'[bottom] override),
 //   then the diffusivity chain nu(Ri), nu_T = Ri > 0 ? nu/Pr : kappa_ca, Ri = g alpha T_z / (u_z^2 + v_z^2) back to the state.
 // Everything is dimensional, with the closure's own dz and dt, as in closure_uvt_kernel; the MLP runs on the adjoint plan with
-// the device functions of the discrete adjoint (run_phase_cached keeping z, mlp_backward_layer).
+// the device functions of the discrete adjoint (mlp_forward_keep, mlp_backward).
 // At relu kinks and at the convective-adjustment switch the derivative is that of the branch the forward evaluated.
 #pragma once
 #include "cpz_adjoint.cuh"
@@ -197,12 +197,7 @@ __global__ void __launch_bounds__(NT, 1) closure_uvt_vjp_kernel(const __grid_con
       __syncthreads();
     }
     if (a.want_mlp) {
-      // MLP forward keeping z and a (the last layer's outputs are not needed: dz_flux is affine in them)
-      for (int p = 0; p < M.n_phase; ++p) {
-        if (M.gemm[M.phase[p].g0].layer == Lmax && M.gemm[M.phase[p].g1 - 1].layer == Lmax) continue;
-        run_phase_cached<CT, NT, WS, true>(M, p, pc, xs, arena, zarena, wsm, a.theta);
-        __syncthreads();
-      }
+      mlp_forward_keep<CT, NT, WS>(M, Lmax, pc, xs, arena, zarena, wsm, a.theta);
       // cotangent of the NN outputs: F = [0; sig (nn_j) + mu - shift; top], dz_flux = D_c F / dz, shift = the first unscaled
       // output, unscaled once more for momentum (:292,301, literal) and as is for temperature (:324)
       for (int i = threadIdx.x; i < 3 * (N - 1) * CT; i += NT) {
@@ -217,10 +212,7 @@ __global__ void __launch_bounds__(NT, 1) closure_uvt_vjp_kernel(const __grid_con
       __syncthreads();
       for (int i = threadIdx.x; i < 3 * N * CT; i += NT) xb[i] = 0.f;
       __syncthreads();
-      for (int l = Lmax; l >= 0; --l) {
-        mlp_backward_layer<WS, CT, NT>(M, l, xs, arena, zarena, xb, wsm, a.theta, gpart);
-        __syncthreads();
-      }
+      mlp_backward<CT, NT, WS>(M, Lmax, xs, arena, zarena, xb, wsm, a.theta, gpart);
     }
     // row stores of u_bar, v_bar, T_bar: the mPP-step part plus the NN-input part unscaled
     for (int i = threadIdx.x; i < 3 * N * CT; i += NT) {
@@ -230,20 +222,7 @@ __global__ void __launch_bounds__(NT, 1) closure_uvt_vjp_kernel(const __grid_con
       a.fbar[q][(size_t)k * a.ncol + col0 + c] = lam[i] + (a.want_mlp ? xb[i] * cd.inv_sig[q] : 0.f);
     }
   }
-  if (!a.want_pgrad) return;
-  // block reduction of the five mPP-parameter sums (fixed order)
-  for (int q = 0; q < 5; ++q) {
-    double vd = pgs[q];
-    for (int o = 16; o > 0; o >>= 1) vd += __shfl_xor_sync(0xffffffffu, vd, o);
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = (float)vd;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      float s = 0.f;
-      for (int wdx = 0; wdx < NT / 32; ++wdx) s += red[wdx];
-      a.lpart[(size_t)blockIdx.x * LP + LP / 2 + q] = s;
-    }
-    __syncthreads();
-  }
+  if (a.want_pgrad) store_pgrad_sums<NT>(pgs, red, a.lpart);
 }
 
 }  // namespace cpz

@@ -6,8 +6,8 @@
 // upper[k] = -r kappa_{k+1}), so A^-T = A^-1: one more Thomas solve with the forward's coefficients. kappa is piecewise
 // constant in T: at the switch the derivative is that of the branch the forward evaluated, as at relu kinks. y, T_mid, dT
 // and Ly enter the forcing additively and drop out.
-// The MLP runs in FP32 SIMT on the adjoint plan with the device functions of the discrete adjoint (run_phase_cached keeping
-// z, mlp_backward_layer); the last layer's forward is skipped, because the forcing is affine in the NN outputs.
+// The MLP runs in FP32 SIMT on the adjoint plan with the device functions of the discrete adjoint (mlp_forward_keep,
+// mlp_backward); the last layer's forward is skipped, because the forcing is affine in the NN outputs.
 #pragma once
 #include "cpz_adjoint.cuh"
 #include "cpz_closure.cuh"
@@ -108,12 +108,7 @@ __global__ void __launch_bounds__(NT, 1) closure_vjp_kernel(const __grid_constan
         }
       }
       __syncthreads();
-      // MLP forward keeping z and a, without the last layer
-      for (int p = 0; p < M.n_phase; ++p) {
-        if (M.gemm[M.phase[p].g0].layer == Lmax && M.gemm[M.phase[p].g1 - 1].layer == Lmax) continue;
-        run_phase_cached<CT, NT, WS, true>(M, p, pc, xs, arena, zarena, wsm, a.theta);
-        __syncthreads();
-      }
+      mlp_forward_keep<CT, NT, WS>(M, Lmax, pc, xs, arena, zarena, wsm, a.theta);
       // cotangent of the NN outputs: wT[j + 1] = sig_wT nn_j + mu_wT, forcing_k = (wT[k + 1] - wT[k]) / dz
       for (int i = threadIdx.x; i < (N - 1) * CT; i += NT) {
         const int j = i / CT, c = i - j * CT;
@@ -122,10 +117,7 @@ __global__ void __launch_bounds__(NT, 1) closure_vjp_kernel(const __grid_constan
       __syncthreads();
       for (int i = threadIdx.x; i < N * CT; i += NT) xb[i] = 0.f;
       __syncthreads();
-      for (int l = Lmax; l >= 0; --l) {
-        mlp_backward_layer<WS, CT, NT>(M, l, xs, arena, zarena, xb, wsm, a.theta, gpart);
-        __syncthreads();
-      }
+      mlp_backward<CT, NT, WS>(M, Lmax, xs, arena, zarena, xb, wsm, a.theta, gpart);
     }
     if (a.T_bar == nullptr) continue;
     // T'bar, then lambda = A^-1 T'bar with the adjustment's coefficients (one thread per column), in place

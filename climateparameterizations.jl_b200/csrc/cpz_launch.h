@@ -24,7 +24,10 @@ bool closure_uses_tc(const cpz_model* m);  // NN-free u/v/T model; 1 = not eligi
 // one line for cpz_model_describe: which forward kernel this model runs on and why
 std::string tc_describe(const cpz_model* m);  // 1 = not eligible, use the SIMT kernel
 int launch_adjoint(cpz_model* m, const AdjArgs& a, int grid);
-// pullback of one RHS evaluation on the adjoint plan (cpz_k_rhs_vjp.cu): persistent grid, one gradient slab per CTA
+// Single-evaluation pullbacks on the adjoint plan (launch_vjp_t): VJP_NT threads per CTA on VJP_CT-column tiles, a persistent
+// grid with one gradient slab per CTA.
+constexpr int VJP_CT = 32, VJP_NT = 256;
+// pullback of one RHS evaluation (cpz_k_rhs_vjp.cu)
 int launch_rhs_vjp(cpz_model* m, const VjpArgs& a, int grid);
 // tensor-core adjoint (cpz_k_adjoint_tc.cu): checkpointing forward solve + reverse sweep; leaves the summed gradient in
 // m->b_red[0,P) and returns the per-tile squared-error sums (stride 8)
@@ -44,10 +47,10 @@ int loss_grad_fc1(cpz_model* m, const float* x0, const float* bcs, const float* 
 int launch_closure(cpz_model* m, const ClosureD& cd, const ClosureArgs& a);
 int launch_closure_uvt(cpz_model* m, const ClosureUvtD& cd, const ClosureUvtArgs& a);
 int launch_closure_uvt_tc(cpz_model* m, const ClosureUvtD& cd, const ClosureUvtArgs& a);  // tcgen05 flavour (cpz_k_tc.cu); 1 = not eligible
-// pullback of the u/v/T closure step on the adjoint plan (cpz_k_closure_uvt_vjp.cu): persistent grid, one gradient slab per CTA
+// pullback of the u/v/T closure step on VJP_CT-column tiles (cpz_k_closure_uvt_vjp.cu)
 struct ClosureUvtVjpArgs;  // cpz_closure_uvt_vjp.cuh
 int launch_closure_uvt_vjp(cpz_model* m, const ClosureUvtD& cd, const ClosureUvtVjpArgs& a, int grid);
-// pullback of the gyre closure step on the adjoint plan (cpz_k_closure_vjp.cu): persistent grid, one gradient slab per CTA
+// pullback of the gyre closure step on VJP_CT-column tiles (cpz_k_closure_vjp.cu)
 struct ClosureVjpArgs;  // cpz_closure_vjp.cuh
 int launch_closure_vjp(cpz_model* m, const ClosureD& cd, const ClosureVjpArgs& a, int grid);
 int launch_reduce_slabs(cpz_model* m, const float* part, int n_slabs, int P, float* out);

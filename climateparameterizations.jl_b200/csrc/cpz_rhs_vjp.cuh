@@ -1,8 +1,8 @@
 // Pullback of the right-hand side (cpz_rhs_vjp): for every column c of a batch
 //   x_bar[c] = (df/dx)^T(x_c) ybar_c,   theta_bar += (df/dtheta)^T(x_c) ybar_c,   p_bar += (df/dp)^T(x_c) ybar_c,
 // p = (nu0, nu_m, dRi, Ric, Pr). This is one reverse stage of adjoint_body (cpz_adjoint.cuh) without the Runge–Kutta
-// bookkeeping, built from the same device functions: MLP forward keeping a and z, faces_vjp, centres_vjp,
-// mlp_backward_layer. It lets a host that runs its own time stepper (adaptive Tsit5 / ROCK4 with InterpolatingAdjoint,
+// bookkeeping, built from the same device functions: mlp_forward_keep, faces_vjp, centres_vjp, mlp_backward.
+// It lets a host that runs its own time stepper (adaptive Tsit5 / ROCK4 with InterpolatingAdjoint,
 // a continuous adjoint) differentiate through cpz_rhs.
 //
 // The boundary fluxes, the diurnal amplitudes and t enter f additively (the two boundary faces of every field), so the
@@ -68,44 +68,19 @@ __global__ void __launch_bounds__(NT, 1) rhs_vjp_kernel(const __grid_constant__ 
         for (int q = 0; q < M.nf; ++q) xb[q * N * CT + i] = 0.f;
     }
     __syncthreads();
-    // MLP forward keeping z and a (the last layer's outputs are not needed: f is linear in them)
-    if (a.want_mlp) {
-      for (int p = 0; p < M.n_phase; ++p) {
-        if (M.gemm[M.phase[p].g0].layer == Lmax && M.gemm[M.phase[p].g1 - 1].layer == Lmax) continue;
-        run_phase_cached<CT, NT, WS, true>(M, p, pc, xs, arena, zarena, wsm, a.theta);
-        __syncthreads();
-      }
-    }
+    if (a.want_mlp) mlp_forward_keep<CT, NT, WS>(M, Lmax, pc, xs, arena, zarena, wsm, a.theta);
     faces_vjp<CT, NT>(M, xs, xb, zarena, gflux, a.want_pgrad ? pgs : nullptr);
     __syncthreads();
     centres_vjp<CT, NT>(M, xb, gflux);
     __syncthreads();
-    if (a.want_mlp) {
-      for (int l = Lmax; l >= 0; --l) {
-        mlp_backward_layer<WS, CT, NT>(M, l, xs, arena, zarena, xb, wsm, a.theta, gpart);
-        __syncthreads();
-      }
-    }
+    if (a.want_mlp) mlp_backward<CT, NT, WS>(M, Lmax, xs, arena, zarena, xb, wsm, a.theta, gpart);
     if (a.xbar != nullptr) {
       store_tile<CT, NT>(xb, xin, a.xbar, (size_t)S, S, col0, a.ncol);
       if (threadIdx.x < CT) bulk_wait_read0();  // xin is the next tile's staging buffer
     }
   }
   if (a.xbar != nullptr && threadIdx.x < CT) bulk_wait0();
-  if (!a.want_pgrad) return;
-  // block reduction of the five mPP-parameter sums (fixed order)
-  for (int q = 0; q < 5; ++q) {
-    double vd = pgs[q];
-    for (int o = 16; o > 0; o >>= 1) vd += __shfl_xor_sync(0xffffffffu, vd, o);
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = (float)vd;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      float s = 0.f;
-      for (int wdx = 0; wdx < NT / 32; ++wdx) s += red[wdx];
-      a.lpart[(size_t)blockIdx.x * LP + LP / 2 + q] = s;
-    }
-    __syncthreads();
-  }
+  if (a.want_pgrad) store_pgrad_sums<NT>(pgs, red, a.lpart);
 }
 
 }  // namespace cpz
