@@ -11,6 +11,7 @@
 #include "cpz_launch.h"
 #include "cpz_closure_uvt_vjp.cuh"
 #include "cpz_closure_vjp.cuh"
+#include "cpz_jvp.cuh"
 
 namespace cpz {
 
@@ -369,6 +370,12 @@ int cpz_model_describe(const cpz_model* m, char* buf, size_t buf_len) {
     pullback("gyre closure-step pullback (cpz_closure_step_vjp)", "closure_vjp_kernel", true);
   s += "solve pullback (cpz_solve_vjp): the cpz_loss_grad kernels above in cotangent mode (the trajectory cotangent replaces the "
        "loss terms at the saved frames; x0 cotangent stored at the end of the reverse sweep)\n";
+  if (m->has_bwd) {
+    snprintf(line, sizeof(line), "tangents (cpz_rhs_jvp, cpz_solve_jvp): rhs_jvp_kernel, solve_jvp_kernel, fp32-simt, 32-column tiles on "
+             "the adjoint plan, weights %s, persistent grid of min(tiles, %d) CTAs; the solve's stage slots k and kdot in a per-CTA "
+             "global scratch\n", m->bwd.M.w_in_smem ? "in shared memory" : "streamed from global memory", m->ctx->sm_count);
+    s += line;
+  }
   if (m->has_small[0]) {
     const int sms = m->ctx->sm_count > 0 ? m->ctx->sm_count : 148;
     snprintf(line, sizeof(line), "small-batch training pass: 4- / 8- / 16-column adjoint tiles while the batch fits one wave (up to %d / %d / %d columns)\n",
@@ -514,6 +521,88 @@ int cpz_rhs_vjp(cpz_model* m, const float* x, const float* bcs, const float* diu
   if (x_bar) CPZ_CUDA(cudaMemcpyAsync(x_bar, m->b_traj.p, ncol * S * sizeof(float), cudaMemcpyDeviceToHost, st));
   if (theta_bar) CPZ_CUDA(cudaMemcpyAsync(theta_bar, m->b_red.p, m->P * sizeof(float), cudaMemcpyDeviceToHost, st));
   if (mpp_bar) CPZ_CUDA(cudaMemcpyAsync(mpp_bar, m->b_out.p, 5 * sizeof(float), cudaMemcpyDeviceToHost, st));
+  CPZ_CUDA(cudaStreamSynchronize(st));
+  return CPZ_OK;
+}
+
+// ---- RHS pushforward ------------------------------------------------------------------------------------------------
+}  // extern "C"
+namespace {
+// Argument checks of cpz_rhs_jvp and cpz_solve_jvp (both flavours); binds the context's device
+int check_jvp_args(cpz_model* m, const char* what, const float* x, const float* bcs, const float* Q, const float* x_dot,
+                   const float* theta_dot, const float* mpp_dot, const float* y_dot, size_t ncol) {
+  int rc = check_model(m);
+  if (rc) return rc;
+  if (ncol == 0) return fail(CPZ_ERR_INVALID, "ncol must be positive");
+  if (!x || !bcs || !y_dot) return fail(CPZ_ERR_INVALID, "null array");
+  if (!x_dot && !theta_dot && !mpp_dot) return fail(CPZ_ERR_INVALID, "%s: no tangent given (x_dot, theta_dot and mpp_dot are all NULL)", what);
+  if ((m->desc.flags & CPZ_FLAG_DIURNAL) && !Q) return fail(CPZ_ERR_INVALID, "diurnal model needs diurnal_Q");
+  if (theta_dot && m->P == 0) return fail(CPZ_ERR_INVALID, "%s: theta_dot given but the model has no parameters", what);
+  if (mpp_dot && (rc = check_mpp_grad(m))) return rc;
+  if (!m->has_bwd) return fail(CPZ_ERR_INVALID, "adjoint plan unavailable: %s", m->bwd_err.c_str());
+  if (ncol > (size_t)INT32_MAX / 512) return fail(CPZ_ERR_INVALID, "ncol too large");
+  return bind_device(m->ctx);
+}
+
+JvpArgs jvp_args(cpz_model* m, const float* x, const float* bcs, const float* Q, const float* x_dot, const float* theta_dot,
+                 const float* mpp_dot, float* y, float* y_dot, size_t ncol, int& grid) {
+  JvpArgs a{};
+  a.theta = m->d_theta; a.theta_dot = theta_dot; a.pdot = mpp_dot; a.x = x; a.xdot = x_dot; a.bcs = bcs; a.Q = Q;
+  a.y = y; a.ydot = y_dot; a.ncol = (int)ncol; a.n_tiles = (int)((ncol + VJP_CT - 1) / VJP_CT);
+  grid = std::min(a.n_tiles, m->ctx->sm_count);
+  return a;
+}
+
+// Host flavours: the inputs go to device staging (x, bcs, Q as upload_inputs does; x_dot in b_tgt, theta_dot in b_red, mpp_dot
+// in b_out), the tangent output to b_traj and the primal output to b_ckpt.
+int stage_jvp_inputs(cpz_model* m, const float* x, const float* bcs, const float* Q, const float* x_dot, const float* theta_dot,
+                     const float* mpp_dot, size_t ncol, size_t out_floats, bool want_y) {
+  int rc;
+  if ((rc = upload_inputs(m, x, bcs, Q, ncol))) return rc;
+  const size_t S = (size_t)m->fwd.M.S;
+  cudaStream_t st = m->ctx->stream;
+  if (x_dot) {
+    if ((rc = ensure(m->b_tgt, ncol * S))) return rc;
+    CPZ_CUDA(cudaMemcpyAsync(m->b_tgt.p, x_dot, ncol * S * sizeof(float), cudaMemcpyHostToDevice, st));
+  }
+  if (theta_dot) {
+    if ((rc = ensure(m->b_red, m->P + 16))) return rc;
+    CPZ_CUDA(cudaMemcpyAsync(m->b_red.p, theta_dot, m->P * sizeof(float), cudaMemcpyHostToDevice, st));
+  }
+  if (mpp_dot) {
+    if ((rc = ensure(m->b_out, 8))) return rc;
+    CPZ_CUDA(cudaMemcpyAsync(m->b_out.p, mpp_dot, 5 * sizeof(float), cudaMemcpyHostToDevice, st));
+  }
+  if ((rc = ensure(m->b_traj, out_floats))) return rc;
+  if (want_y && (rc = ensure(m->b_ckpt, out_floats))) return rc;
+  return CPZ_OK;
+}
+}  // namespace
+extern "C" {
+
+int cpz_rhs_jvp_dev(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, const float* x_dot,
+                    const float* theta_dot, const float* mpp_dot, float* dxdt, float* dxdt_dot, size_t ncol) {
+  int rc = check_jvp_args(m, "rhs_jvp", x, bcs, diurnal_Q, x_dot, theta_dot, mpp_dot, dxdt_dot, ncol);
+  if (rc) return rc;
+  int grid = 0;
+  JvpArgs a = jvp_args(m, x, bcs, diurnal_Q, x_dot, theta_dot, mpp_dot, dxdt, dxdt_dot, ncol, grid);
+  a.t = t;
+  return launch_rhs_jvp(m, a, grid);
+}
+
+int cpz_rhs_jvp(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, const float* x_dot,
+                const float* theta_dot, const float* mpp_dot, float* dxdt, float* dxdt_dot, size_t ncol) {
+  int rc = check_jvp_args(m, "rhs_jvp", x, bcs, diurnal_Q, x_dot, theta_dot, mpp_dot, dxdt_dot, ncol);
+  if (rc) return rc;
+  const size_t n = ncol * (size_t)m->fwd.M.S;
+  if ((rc = stage_jvp_inputs(m, x, bcs, diurnal_Q, x_dot, theta_dot, mpp_dot, ncol, n, dxdt != nullptr))) return rc;
+  if ((rc = cpz_rhs_jvp_dev(m, m->b_x0.p, m->b_bcs.p, diurnal_Q ? m->b_q.p : nullptr, t, x_dot ? m->b_tgt.p : nullptr,
+                            theta_dot ? m->b_red.p : nullptr, mpp_dot ? m->b_out.p : nullptr, dxdt ? m->b_ckpt.p : nullptr,
+                            m->b_traj.p, ncol)))
+    return rc;
+  cudaStream_t st = m->ctx->stream;
+  CPZ_CUDA(cudaMemcpyAsync(dxdt_dot, m->b_traj.p, n * sizeof(float), cudaMemcpyDeviceToHost, st));
+  if (dxdt) CPZ_CUDA(cudaMemcpyAsync(dxdt, m->b_ckpt.p, n * sizeof(float), cudaMemcpyDeviceToHost, st));
   CPZ_CUDA(cudaStreamSynchronize(st));
   return CPZ_OK;
 }

@@ -53,6 +53,10 @@ int launch_closure_uvt_vjp(cpz_model* m, const ClosureUvtD& cd, const ClosureUvt
 // pullback of the gyre closure step on VJP_CT-column tiles (cpz_k_closure_vjp.cu)
 struct ClosureVjpArgs;  // cpz_closure_vjp.cuh
 int launch_closure_vjp(cpz_model* m, const ClosureD& cd, const ClosureVjpArgs& a, int grid);
+// pushforwards of one RHS evaluation and of the solve on VJP_CT-column tiles (cpz_k_jvp.cu)
+struct JvpArgs;  // cpz_jvp.cuh
+int launch_rhs_jvp(cpz_model* m, const JvpArgs& a, int grid);
+int launch_solve_jvp(cpz_model* m, const JvpArgs& a, int grid);
 int launch_reduce_slabs(cpz_model* m, const float* part, int n_slabs, int P, float* out);
 int launch_pack_loss(cpz_model* m, const float* lpart, int n_slabs, int stride, float ncol, float* pack_tail);
 int launch_finalize_loss(cpz_model* m, const float* pack_tail, const float* w6, float inv_prof, float inv_grad, float* loss_out);

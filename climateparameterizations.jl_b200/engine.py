@@ -21,7 +21,8 @@ EXPORTS = [
     "cpz_rhs_dev", "cpz_rhs_vjp", "cpz_rhs_vjp_dev", "cpz_predict_flux", "cpz_predict_flux_dev", "cpz_solve", "cpz_solve_dev", "cpz_solve_vjp", "cpz_solve_vjp_dev", "cpz_loss_grad", "cpz_loss_grad_dev", "cpz_train_step",
     "cpz_train_step_dev", "cpz_set_mpp_params", "cpz_get_mpp_params", "cpz_loss_grad_mpp", "cpz_loss_grad_mpp_dev", "cpz_adam_get_state", "cpz_adam_set_state", "cpz_closure_step", "cpz_closure_step_dev",
     "cpz_sizeof_closure_uvt_desc", "cpz_closure_step_uvt", "cpz_closure_step_uvt_dev", "cpz_closure_step_uvt_vjp",
-    "cpz_closure_step_uvt_vjp_dev", "cpz_closure_step_vjp", "cpz_closure_step_vjp_dev",
+    "cpz_closure_step_uvt_vjp_dev", "cpz_closure_step_vjp", "cpz_closure_step_vjp_dev", "cpz_rhs_jvp", "cpz_rhs_jvp_dev",
+    "cpz_solve_jvp", "cpz_solve_jvp_dev",
 ]
 
 ALLREDUCE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p)
@@ -75,6 +76,10 @@ def lib() -> C.CDLL:
         getattr(L, name).argtypes = [vp, vp, vp, vp, vp, sz]
     for name in ("cpz_solve_vjp", "cpz_solve_vjp_dev"):
         getattr(L, name).argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, sz]
+    for name in ("cpz_rhs_jvp", "cpz_rhs_jvp_dev"):
+        getattr(L, name).argtypes = [vp, vp, vp, vp, f32, vp, vp, vp, vp, vp, sz]
+    for name in ("cpz_solve_jvp", "cpz_solve_jvp_dev"):
+        getattr(L, name).argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, sz]
     for name in ("cpz_loss_grad", "cpz_loss_grad_dev"):
         getattr(L, name).argtypes = [vp, vp, vp, vp, vp, sz, vp, vp, vp]
     for name in ("cpz_loss_grad_mpp", "cpz_loss_grad_mpp_dev"):
@@ -271,6 +276,22 @@ class Model:
                                  ncol))
         return xb, tb, pb
 
+    def rhs_jvp(self, x, bcs, x_dot=None, theta_dot=None, mpp_dot=None, t: float = 0.0, Q=None, want_dxdt: bool = True):
+        """Pushforward of rhs() at x — cpz_rhs_jvp: (dxdt [ncol, S] or None, dxdt_dot [ncol, S]) for the tangents x_dot
+        [ncol, S], theta_dot [P] and mpp_dot [5] wrt (nu0, nu_m, dRi, Ric, Pr); a tangent that is None counts as zero."""
+        x = _np(x)
+        ncol = x.shape[0]
+        bcs = _np(bcs, (ncol, self.desc.n_bc))
+        Q = None if Q is None else _np(Q, (ncol,))
+        xd = None if x_dot is None else _np(x_dot, x.shape)
+        td = None if theta_dot is None else _np(theta_dot, (self.P,))
+        pd = None if mpp_dot is None else _np(mpp_dot, (5,))
+        y = np.empty_like(x) if want_dxdt else None
+        yd = np.empty_like(x)
+        _check(lib().cpz_rhs_jvp(self._h, _ptr(x), _ptr(bcs), _ptr(Q), float(t), _ptr(xd), _ptr(td), _ptr(pd), _ptr(y), _ptr(yd),
+                                 ncol))
+        return y, yd
+
     def predict_flux(self, x, bcs, t: float = 0.0, Q=None) -> np.ndarray:
         """Total face fluxes [ncol, n_fields, Nz+1] (scaled) of one RHS evaluation — cpz_predict_flux."""
         x = _np(x)
@@ -304,6 +325,23 @@ class Model:
         pb = np.empty(5, dtype=np.float32) if want_mpp else None
         _check(lib().cpz_solve_vjp(self._h, _ptr(x0), _ptr(bcs), _ptr(Q), _ptr(tb_in), _ptr(xb), _ptr(tb), _ptr(pb), ncol))
         return xb, tb, pb
+
+    def solve_jvp(self, x0, bcs, x0_dot=None, theta_dot=None, mpp_dot=None, Q=None, want_traj: bool = True):
+        """Pushforward of solve() at x0 (the tangent-linear model) — cpz_solve_jvp: (traj or None, traj_dot), both
+        [ncol, n_saved, S], for the tangents x0_dot [ncol, S], theta_dot [P] and mpp_dot [5]; a tangent that is None counts
+        as zero. traj is the FP32 pass's primal trajectory."""
+        x0 = _np(x0)
+        ncol = x0.shape[0]
+        bcs = _np(bcs, (ncol, self.desc.n_bc))
+        Q = None if Q is None else _np(Q, (ncol,))
+        xd = None if x0_dot is None else _np(x0_dot, x0.shape)
+        td = None if theta_dot is None else _np(theta_dot, (self.P,))
+        pd = None if mpp_dot is None else _np(mpp_dot, (5,))
+        shape = (ncol, self.n_saved, self.desc.S)
+        y = np.empty(shape, dtype=np.float32) if want_traj else None
+        yd = np.empty(shape, dtype=np.float32)
+        _check(lib().cpz_solve_jvp(self._h, _ptr(x0), _ptr(bcs), _ptr(Q), _ptr(xd), _ptr(td), _ptr(pd), _ptr(y), _ptr(yd), ncol))
+        return y, yd
 
     def loss_grad(self, x0, bcs, targets, loss_w, Q=None, want_grad: bool = True):
         x0 = _np(x0)
@@ -435,6 +473,13 @@ class Model:
         _check(lib().cpz_rhs_vjp_dev(self._h, _ptr(x), _ptr(bcs), _ptr(Q), float(t), _ptr(dxdt_bar), _ptr(x_bar),
                                      _ptr(theta_bar), _ptr(mpp_bar), ncol))
 
+    def rhs_jvp_dev(self, x, bcs, dxdt_dot, x_dot=None, theta_dot=None, mpp_dot=None, dxdt=None, t: float = 0.0, Q=None,
+                    ncol: Optional[int] = None) -> None:
+        """cpz_rhs_jvp_dev: dxdt_dot [ncol, S] (and dxdt when given) are overwritten; a tangent that is None counts as zero."""
+        ncol = ncol if ncol is not None else x.shape[0]
+        _check(lib().cpz_rhs_jvp_dev(self._h, _ptr(x), _ptr(bcs), _ptr(Q), float(t), _ptr(x_dot), _ptr(theta_dot), _ptr(mpp_dot),
+                                     _ptr(dxdt), _ptr(dxdt_dot), ncol))
+
     def solve_dev(self, x0, bcs, traj, Q=None, ncol: Optional[int] = None) -> None:
         ncol = ncol if ncol is not None else x0.shape[0]
         _check(lib().cpz_solve_dev(self._h, _ptr(x0), _ptr(bcs), _ptr(Q), _ptr(traj), ncol))
@@ -445,6 +490,14 @@ class Model:
         ncol = ncol if ncol is not None else x0.shape[0]
         _check(lib().cpz_solve_vjp_dev(self._h, _ptr(x0), _ptr(bcs), _ptr(Q), _ptr(traj_bar), _ptr(x0_bar), _ptr(theta_bar),
                                        _ptr(mpp_bar), ncol))
+
+    def solve_jvp_dev(self, x0, bcs, traj_dot, x0_dot=None, theta_dot=None, mpp_dot=None, traj=None, Q=None,
+                      ncol: Optional[int] = None) -> None:
+        """cpz_solve_jvp_dev: traj_dot [ncol, n_saved, S] (and traj when given) are overwritten; a tangent that is None counts
+        as zero."""
+        ncol = ncol if ncol is not None else x0.shape[0]
+        _check(lib().cpz_solve_jvp_dev(self._h, _ptr(x0), _ptr(bcs), _ptr(Q), _ptr(x0_dot), _ptr(theta_dot), _ptr(mpp_dot),
+                                       _ptr(traj), _ptr(traj_dot), ncol))
 
     def loss_grad_dev(self, x0, bcs, targets, loss_w, loss_out, grad_out, Q=None, ncol: Optional[int] = None) -> None:
         ncol = ncol if ncol is not None else x0.shape[0]

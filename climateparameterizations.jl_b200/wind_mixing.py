@@ -502,3 +502,92 @@ def _closure_autograd_function():
 
     return ClosureStepUvt
 
+
+
+def solve_autograd(model: engine.Model, theta, x0, bcs, Q=None, p=None):
+    """The batched solve (cpz_solve_dev) as a torch autograd node for any model, u/v/T or T-only: traj [ncol, n_saved, S] of
+    CUDA float32 x0 [ncol, S] and bcs [ncol, n_bc] (and diurnal amplitudes Q [ncol]) on the model's device. `theta` ([P]
+    tensor) is copied into the model first; `p` (optional [5] tensor (nu0, nu_m, dRi, Ric, Pr)) sets the mPP parameters.
+    Reverse mode runs cpz_solve_vjp_dev (theta, x0 and p receive their cotangents), forward mode (torch.autograd.forward_ad,
+    torch.func.jvp) cpz_solve_jvp_dev with the tangents of theta, x0 and p. bcs and Q are data: they get no derivative."""
+    global _SOLVE
+    if _SOLVE is None:  # built on first use: importing this module does not import torch
+        _SOLVE = _solve_autograd_function()
+    return _SOLVE.apply(model, theta, x0, bcs, Q, p)
+
+
+_SOLVE = None
+
+
+def _solve_autograd_function():
+    import torch
+    from torch._C import _functorch
+    from torch._functorch.pyfunctorch import temporarily_clear_interpreter_stack
+
+    # Under torch.func transforms the tensors a Function sees (and the ones it allocates) are functorch wrappers without
+    # storage; the engine needs raw device pointers, so every engine call runs on the unwrapped tensors with the transform
+    # stack cleared (torch's own private hooks for this: there is no public one in this torch version).
+    def raw(a):
+        while a is not None and _functorch.is_functorch_wrapped_tensor(a):
+            a = _functorch.get_unwrapped(a)
+        return None if a is None else a.detach().float().contiguous()
+
+    class Solve(torch.autograd.Function):
+        @staticmethod
+        def forward(model, theta, x0, bcs, Q, p):
+            with temporarily_clear_interpreter_stack():
+                if model.P > 0:
+                    model.set_theta(raw(theta).cpu().numpy())
+                if p is not None:
+                    model.set_mpp_params(*(float(v) for v in raw(p).cpu()))
+                x0, bcs, Q = raw(x0), raw(bcs), raw(Q)
+                traj = torch.empty((x0.shape[0], model.n_saved, model.desc.S), device=x0.device)
+                torch.cuda.synchronize(x0.device)
+                model.solve_dev(x0, bcs, traj, Q=Q)
+                model.ctx.synchronize()
+            return traj
+
+        @staticmethod
+        def setup_context(fctx, inputs, output):
+            model, theta, x0, bcs, Q, p = inputs
+            fctx.model, fctx.has_p = model, p is not None
+            fctx.meta = [(a.dtype, a.device) if a is not None else None for a in (theta, x0, p)]
+            fctx.data = (x0, bcs, Q)
+
+        @staticmethod
+        def backward(fctx, traj_bar):
+            m = fctx.model
+            want = fctx.needs_input_grad
+            with temporarily_clear_interpreter_stack():
+                x0, bcs, Q = (raw(a) for a in fctx.data)
+                xb = torch.empty_like(x0) if want[2] else None
+                tb = torch.empty(m.P, device=x0.device) if want[1] and m.P > 0 else None
+                pb = torch.empty(5, device=x0.device) if want[5] and fctx.has_p else None
+                if xb is None and tb is None and pb is None:
+                    return None, None, None, None, None, None
+                torch.cuda.synchronize(x0.device)
+                m.solve_vjp_dev(x0, bcs, raw(traj_bar), x0_bar=xb, theta_bar=tb, mpp_bar=pb, Q=Q)
+                m.ctx.synchronize()
+            out = [tb, xb, pb]
+            for i, meta in enumerate(fctx.meta):
+                if out[i] is not None:
+                    out[i] = out[i].to(dtype=meta[0], device=meta[1])
+            return None, out[0], out[1], None, None, out[2]
+
+        @staticmethod
+        def jvp(fctx, model_t, theta_t, x0_t, bcs_t, Q_t, p_t):
+            m = fctx.model
+            with temporarily_clear_interpreter_stack():
+                x0, bcs, Q = (raw(a) for a in fctx.data)
+                dev = x0.device
+                td = raw(theta_t).to(dev) if (theta_t is not None and m.P > 0) else None
+                xd = None if x0_t is None else raw(x0_t).to(dev)
+                pd = raw(p_t).to(dev) if (p_t is not None and fctx.has_p) else None
+                traj_dot = torch.zeros((x0.shape[0], m.n_saved, m.desc.S), device=dev)
+                if xd is not None or td is not None or pd is not None:
+                    torch.cuda.synchronize(dev)
+                    m.solve_jvp_dev(x0, bcs, traj_dot, x0_dot=xd, theta_dot=td, mpp_dot=pd, Q=Q)
+                    m.ctx.synchronize()
+            return traj_dot
+
+    return Solve

@@ -230,6 +230,32 @@ int cpz_solve_vjp(cpz_model* m, const float* x0, const float* bcs, const float* 
 int cpz_solve_vjp_dev(cpz_model* m, const float* x0, const float* bcs, const float* diurnal_Q, const float* traj_bar,
                       float* x0_bar, float* theta_bar, float* mpp_bar, size_t ncol);
 
+/* ---- S1 / S2 pushforwards: JVPs of f(x, p, t) and of the solve ------------------------------------------------------ */
+/* Forward-mode derivatives for hosts that need J v: Rosenbrock / Newton-Krylov integrators (J v per column, or the dense
+ * S x S Jacobian of a column from S replicated columns with unit tangents), forward sensitivities wrt few parameters, the
+ * tangent-linear model. With f_c = what cpz_rhs returns and traj_c = what cpz_solve writes for column c on the same inputs:
+ *   dxdt_dot[c] = (df_c/dx) x_dot[c] + (df_c/dtheta) theta_dot + (df_c/dp) mpp_dot                     [ncol][nf*Nz]
+ *   traj_dot[c] = (dtraj_c/dx0) x0_dot[c] + (dtraj_c/dtheta) theta_dot + (dtraj_c/dp) mpp_dot          [ncol][n_saved][nf*Nz]
+ * Tangents: x_dot / x0_dot [ncol][nf*Nz], theta_dot [P] in Flux.destructure order, mpp_dot [5] wrt p = (nu0, nu_m, dRi, Ric,
+ * Pr) unscaled (the meaning cpz_loss_grad_mpp uses). A NULL tangent counts as zero; at least one must be given. theta_dot
+ * is refused when P = 0, mpp_dot where cpz_loss_grad_mpp refuses it. dxdt_dot / traj_dot are required; dxdt / traj are
+ * optional and receive the primal result of the same pass. Outputs are overwritten, not accumulated. ncol must be positive.
+ * With CPZ_FLAG_IMPLICIT_DIFFUSION cpz_rhs_jvp differentiates the explicit part cpz_rhs returns (mpp_dot contributes 0), and
+ * cpz_solve_jvp the whole split step, backward-Euler solve included. At relu kinks, the convective-adjustment switch and
+ * CPZ_FLAG_CA_LITERAL_U the derivative of the evaluated branch is taken, as in the pullbacks. Nothing is summed over
+ * columns: a column's result depends only on its own inputs (bitwise batch invariance); the allreduce hook is not called
+ * and there is no non-finite reporting. Both run FP32 SIMT kernels on the adjoint plan (a model without one is refused with
+ * the planner's reason); traj therefore comes from the FP32 pass and differs from cpz_solve's 3xTF32 result for the
+ * production nets by rounding. */
+int cpz_rhs_jvp(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, const float* x_dot,
+                const float* theta_dot, const float* mpp_dot, float* dxdt, float* dxdt_dot, size_t ncol);
+int cpz_rhs_jvp_dev(cpz_model* m, const float* x, const float* bcs, const float* diurnal_Q, float t, const float* x_dot,
+                    const float* theta_dot, const float* mpp_dot, float* dxdt, float* dxdt_dot, size_t ncol);
+int cpz_solve_jvp(cpz_model* m, const float* x0, const float* bcs, const float* diurnal_Q, const float* x0_dot,
+                  const float* theta_dot, const float* mpp_dot, float* traj, float* traj_dot, size_t ncol);
+int cpz_solve_jvp_dev(cpz_model* m, const float* x0, const float* bcs, const float* diurnal_Q, const float* x0_dot,
+                      const float* theta_dot, const float* mpp_dot, float* traj, float* traj_dot, size_t ncol);
+
 /* ---- S3: objective and gradient ------------------------------------------------------------- */
 /* replaces loss_NDE / loss_gradient_NDE + Zygote gradient (NDE_training.jl:290-333; loss.jl:1-42) and
  * nde_loss (free_convection/src/training.jl:55-62).
