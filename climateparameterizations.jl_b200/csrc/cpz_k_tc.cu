@@ -50,19 +50,10 @@ bool tc_plan(const cpz_model* m, TcD& T, std::string& why) {
   T.act1 = n0.act[0]; T.act2 = n0.act[1]; T.act3 = n0.act[2];
   if (3 * T.h1 > 160 || T.h2 > 32 || T.h1 < 1 || T.h2 < 1) { why = "hidden widths outside 3*h1 <= 160, h2 <= 32"; return false; }
   T.n1b = 3 * T.h1 > 128 ? 3 * T.h1 - 128 : 0;
-  // K windows: net q's inputs are operand rows width*q.. ; a window starts on a 4-row chunk and spans 8*steps rows
-  int need2 = 0, need3 = 0;
-  for (int q = 0; q < 3; ++q) {
-    T.k2_start[q] = (T.h1 * q) & ~3; T.k3_start[q] = (T.h2 * q) & ~3;
-    need2 = std::max(need2, T.h1 * q + T.h1 - T.k2_start[q]);
-    need3 = std::max(need3, T.h2 * q + T.h2 - T.k3_start[q]);
-  }
-  if (need2 > 8 * TC_K2S) { why = "layer-2 window"; return false; }
-  T.k3_steps = need3 <= 24 ? 3 : 4;
-  if (need3 > 32) { why = "layer-3 window needs more than 4 K steps"; return false; }
-  // operand rows: the layer-1 epilogue writes rows 0..127 unconditionally and rows 128..128+n1b of the quadrant-3 block
-  T.h1_rows = (std::max(T.k2_start[2] + 8 * TC_K2S, 160) + 7) & ~7;
-  T.h2_rows = (T.k3_start[2] + 8 * T.k3_steps + 7) & ~7;
+  // the H1 / H2 planes hold one net's units in K (h1 <= 53 <= 8 * TC_K2S): every K row a layer-2 / layer-3 chain reads
+  T.k3_steps = T.h2 <= 24 ? 3 : 4;
+  T.h1_rows = 8 * TC_K2S;
+  T.h2_rows = 8 * T.k3_steps;
   const int K2 = 8 * TC_K2S, K3 = 8 * T.k3_steps;
   if (2 * K2 + 2 * K3 > 192) { why = "layer-2/3 stacks exceed the 192 free TMEM columns"; return false; }
   T.c_a2hi = 192; T.c_a2lo = 192 + K2; T.c_a3hi = 192 + 2 * K2; T.c_a3lo = 192 + 2 * K2 + K3;
@@ -95,9 +86,9 @@ std::string tc_describe(const cpz_model* m) {
   const TcSmem L = tc_smem_layout(T, m->tab.n_stages);
   snprintf(line, sizeof(line),
            "forward kernel: tcgen05 3xTF32 (weights in TMEM; %d column groups x %d columns, %d threads; layer-1 rows %d+%d, "
-           "layer-2 %d K steps, layer-3 %d K steps; MMAs per RHS and group %d; smem %d B)\n",
+           "layer-2 %d K steps, layer-3 %d K steps, the three nets in one N=48 chain; MMAs per RHS and group %d; smem %d B)\n",
            TC_NG, TC_GN, TC_NT, 3 * T.h1 - T.n1b, T.n1b, TC_K2S, T.k3_steps,
-           36 * (T.n1b > 0 ? 2 : 1) + 9 * TC_K2S + 9 * T.k3_steps, L.total);
+           36 * (T.n1b > 0 ? 2 : 1) + 3 * TC_K2S + 3 * T.k3_steps, L.total);
   return line;
 }
 

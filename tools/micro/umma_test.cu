@@ -3,7 +3,8 @@
 //   T2  TS  same product with A staged in TMEM by tcgen05.st (lane = row, column = k)
 //   T3  SS  quadrant placement: A descriptor start moved back by q*4*SBO so a 32-row A lands in TMEM lanes 32q..32q+31
 //   T4  3xTF32 accuracy on random FP32 data (hi/lo split, three accumulating MMAs)
-//   T5  timings (clock64): MMA chains at N=16/32 (SS and TS), commit->mbarrier round trip, tcgen05.ld
+//   T5  timings (clock64): MMA chains at N=16/32 (SS and TS), TS at N=16/32/48/64, commit->mbarrier round trip, tcgen05.ld
+//   T8  address probe of the N=48 B plane of the forward kernel's layers 2/3 (SBO=128, LBO=6*128+16=784), checked on the host
 // build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o umma_test umma_test.cu
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -92,7 +93,7 @@ struct Out {
   float d2[128 * 32];   // T2
   float d3[128 * 32];   // T3: three nets, net q in lanes 32q.., columns 0..15 of region q -> stored [lane][q*... ] see below
   float d4[128 * 32];   // T4
-  long long t[16];
+  long long t[32];
 };
 
 // Ahi/Alo: [128][96] row-major (m,k). Bhi/Blo: [32][96] (n,k). A3: [3][32][24]; B3: [16][24]
@@ -364,6 +365,39 @@ __global__ void __launch_bounds__(128, 1) umma_kernel(const float* __restrict__ 
     tc_before();
     __syncthreads();
   }
+  // ---------------- T8: the same probe at N=48 with the layer-2/3 B plane of the forward kernel (SBO=128, LBO=784)
+  if (test == 8) {
+    {
+      const int m = warp * 32 + lane;
+      float v[8];
+      for (int j = 0; j < 8; ++j) v[j] = (m == j) ? 1.f : 0.f;
+      tmem_st8(tb + ((uint32_t)(warp * 32) << 16), v);
+      asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+    }
+    for (int i = tid; i < 8192; i += 128) reinterpret_cast<float*>(sB)[i] = (float)i;
+    fence_async();
+    tc_before();
+    __syncthreads();
+    const uint32_t D8 = tb + 400;
+    if (warp == 0) {
+      tc_after();
+      uint32_t el = 0;
+      asm volatile("{\n\t.reg .b32 rx;\n\t.reg .pred px;\n\telect.sync rx|px, 0xffffffff;\n\t@px mov.s32 %0, 1;\n\t}" : "+r"(el));
+      if (el) { mma_ts(D8, tb, make_desc(smem_u32(sB), b_lbo(48), B_SBO), make_idesc(128, 48), 0); mma_commit(&bar); }
+      __syncwarp();
+    }
+    mbar_wait(&bar, parity); parity ^= 1;
+    tc_after();
+    {
+      float v[32];
+      tmem_ld32(D8 + ((uint32_t)(warp * 32) << 16), v);
+      for (int n = 0; n < 32; ++n) out->d1[(warp * 32 + lane) * 32 + n] = v[n];
+      tmem_ld32(D8 + 32 + ((uint32_t)(warp * 32) << 16), v);
+      for (int n = 0; n < 32; ++n) out->d2[(warp * 32 + lane) * 32 + n] = v[n];
+    }
+    tc_before();
+    __syncthreads();
+  }
   // ---------------- T5: timings (warp-uniform issue + elect.sync, descriptors advanced by adds) ----------------
   if (test == 5) {
   if (warp == 0) {
@@ -390,7 +424,7 @@ __global__ void __launch_bounds__(128, 1) umma_kernel(const float* __restrict__ 
       long long c1 = clock64();                                                             \
       mbar_wait(&bar, parity); parity ^= 1;                                                 \
       long long c2 = clock64();                                                             \
-      if (lane == 0) { out->t[slot] = c2 - c0; out->t[slot + 8] = c1 - c0; }               \
+      if (lane == 0) { out->t[slot] = c2 - c0; out->t[slot + 16] = c1 - c0; }              \
     }
     TIME_CHAIN(1, 6, 32, 0)
     TIME_CHAIN(2, 6, 32, 1)
@@ -399,6 +433,7 @@ __global__ void __launch_bounds__(128, 1) umma_kernel(const float* __restrict__ 
     TIME_CHAIN(5, 12, 16, 1)
     TIME_CHAIN(6, 12, 32, 1)
     TIME_CHAIN(7, 12, 64, 1)
+    TIME_CHAIN(9, 12, 48, 1)
     {
       const uint32_t id = make_idesc(128, 16);
       long long c0 = clock64();
@@ -512,6 +547,20 @@ int main(int argc, char** argv) {
       printf("\n");
     }
   }
+  if (test == 8) {
+    // D[m][n] = word index of B(n, k=m); expected byte(n, k) = (n/8)*128 + (n%8)*16 + (k/4)*784 + (k%4)*4
+    int bad = 0;
+    printf("T8 probe (byte offsets of B(n,k), N=48, LBO=784 SBO=128): rows k=0..7, cols n=0..47\n");
+    for (int m = 0; m < 8; ++m) {
+      for (int n = 0; n < 48; ++n) {
+        const int got = (int)((n < 32 ? o->d1[m * 32 + n] : o->d2[m * 32 + n - 32]) * 4);
+        bad += got != (int)kmaj_off(n, m, B_SBO, b_lbo(48));
+        printf("%5d", got);
+      }
+      printf("\n");
+    }
+    printf("T8 N=48 layout: %d of 384 offsets differ from (n/8)*128 + (n%%8)*16 + (k/4)*784 + (k%%4)*4\n", bad);
+  }
   if (test == 6) {
     double e6 = 0;
     for (int m = 0; m < 128; ++m)
@@ -522,7 +571,9 @@ int main(int argc, char** argv) {
       }
     printf("T6 TS + MN-major B window: max abs err %.3g\n", e6);
   }
-  printf("T5 cycles total(issue-only): 72 SS N32 %lld(%lld) | 72 TS N32 %lld(%lld) | 72 SS N16 %lld(%lld) | 72 TS N16 %lld(%lld) | 144 TS N16 %lld(%lld) | 144 TS N32 %lld(%lld) | 144 TS N64 %lld(%lld) | 1 MMA rt %lld | ld.x32 %lld\n",
-         o->t[1], o->t[9], o->t[2], o->t[10], o->t[3], o->t[11], o->t[4], o->t[12], o->t[5], o->t[13], o->t[6], o->t[14], o->t[7], o->t[15], o->t[0], o->t[8]);
+  printf("T5 cycles total(issue-only): 72 SS N32 %lld(%lld) | 72 TS N32 %lld(%lld) | 72 SS N16 %lld(%lld) | 72 TS N16 %lld(%lld) | 144 TS N16 %lld(%lld) | 144 TS N32 %lld(%lld) | 144 TS N48 %lld(%lld) | 144 TS N64 %lld(%lld) | 1 MMA rt %lld | ld.x32 %lld\n",
+         o->t[1], o->t[17], o->t[2], o->t[18], o->t[3], o->t[19], o->t[4], o->t[20], o->t[5], o->t[21], o->t[6], o->t[22], o->t[9], o->t[25], o->t[7], o->t[23], o->t[0], o->t[8]);
+  if (test == 5)
+    printf("T5 cycles per TS MMA (144 back to back): N16 %.1f | N32 %.1f | N48 %.1f | N64 %.1f\n", o->t[5] / 144.0, o->t[6] / 144.0, o->t[9] / 144.0, o->t[7] / 144.0);
   return 0;
 }
