@@ -22,7 +22,7 @@ import make_fullsize  # noqa: E402  (puts the repository and tests/ on sys.path,
 from make_fullsize import W3, bench_targets, load, save  # noqa: E402,F401
 from cpz_b200 import synthetic as syn  # noqa: E402
 from cpz_b200.desc import RHS_TRAIN  # noqa: E402
-from util import oracle_loss_grad  # noqa: E402
+from util import SPREAD_SEEDS, oracle_loss_grad, theta_blocks, ulp_nudge  # noqa: E402
 
 CHUNK = 300
 
@@ -52,12 +52,20 @@ def chunked_loss_grad(d, th, x0, bcs, tgt, w, dtype):
     return tot, comps, g
 
 
+def block_floors(d, th, x0, bcs, tgt, g, g32):
+    """Per (net, layer, W/b) block of theta (util.theta_blocks order): the largest relative L2 error of the FP32-oracle gradient
+    over its plain run and runs at x0 nudged by one ulp (util.assert_blocks' spread floor; the first two SPREAD_SEEDS, as each
+    run takes minutes here)."""
+    runs = [g32] + [chunked_loss_grad(d, th, ulp_nudge(x0, s), bcs, tgt, W3, torch.float32)[2] for s in SPREAD_SEEDS[:2]]
+    return np.array([max(np.linalg.norm(r[sl] - g[sl]) for r in runs) / np.linalg.norm(g[sl]) for _, sl in theta_blocks(d)])
+
+
 def adjoint_case(name):
     d, th, x0, bcs, tgt = case_inputs(name)
     tot, comps, g = chunked_loss_grad(d, th, x0, bcs, tgt, W3, torch.float64)
     tot32, _, g32 = chunked_loss_grad(d, th, x0, bcs, tgt, W3, torch.float32)
     return dict(loss=np.concatenate([comps, [tot]]), grad=g, floor_grad=np.linalg.norm(g32 - g) / np.linalg.norm(g),
-                floor_loss=abs(tot32 - tot) / abs(tot))
+                floor_loss=abs(tot32 - tot) / abs(tot), floor_grad_blocks=block_floors(d, th, x0, bcs, tgt, g, g32))
 
 
 CASES = {name: (lambda name=name: adjoint_case(name)) for name in SHAPES}

@@ -10,7 +10,7 @@ from cpz_b200 import engine, synthetic as syn
 from cpz_b200.desc import (FLAG_CA, FLAG_DIURNAL, FLAG_MPP, FLAG_SMOOTH_NN, FLAG_SMOOTH_RI, FLAG_ZERO_WEIGHTS, RHS_INFER,
                            RHS_TRAIN)
 from oracle import nde
-from util import oracle_loss_grad, oracle_solve, rel_inf, t64
+from util import assert_blocks, fp32_spread, oracle_loss_grad, oracle_solve, rel_inf, t64, theta_blocks, ulp_nudge
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -49,6 +49,8 @@ def _check(ctx, d, th, ncol, w, use_q=False, th_target=None):
     # the min(0,.) / stability switches flip under rounding); there the CUDA result must be at least as close to the
     # FP64 oracle as the FP32 oracle is.
     assert e_g <= max(TOL, f_g), (e_g, f_g)
+    spread = fp32_spread(lambda s: oracle_loss_grad(d, th, ulp_nudge(x0, s), bcs, tgt, w, Q, dtype=torch.float32)[2])
+    assert_blocks("grad", grad, g, g32, theta_blocks(d), TOL, norm="l2", spread=spread)
     assert abs(loss_only[6] - tot) / abs(tot) <= TOL
     return loss, grad
 

@@ -8,7 +8,7 @@ import torch
 
 from cpz_b200 import engine, synthetic as syn
 from cpz_b200.desc import FLAG_CA, FLAG_DIURNAL, FLAG_MPP, FLAG_ZERO_WEIGHTS, RHS_INFER, RHS_TRAIN
-from util import oracle_loss_grad, oracle_solve
+from util import assert_blocks, fp32_spread, oracle_loss_grad, oracle_solve, theta_blocks, ulp_nudge
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -67,6 +67,9 @@ def test_tc_adjoint_matches_the_oracle(ctx, case, split, monkeypatch):
     assert np.isfinite(grad).all() and np.linalg.norm(g) > 0
     assert e_l <= TOL and e_c <= TOL
     assert e_g <= max(TOL, f_g) and e_s <= max(TOL, f_g)
+    spread = fp32_spread(lambda s: oracle_loss_grad(d, th, ulp_nudge(x0, s), bcs, tgt, W_GRAD, Q, dtype=torch.float32)[2])
+    assert_blocks("tc adjoint grad", grad, g, g32, theta_blocks(d), TOL, norm="l2", spread=spread)
+    assert_blocks("fp32 simt adjoint grad", grad_s, g, g32, theta_blocks(d), TOL, norm="l2", spread=spread)
     assert abs(loss[6] - loss_s[6]) <= 1e-5 * abs(loss_s[6])
 
 

@@ -34,7 +34,8 @@ from cpz_b200 import engine, synthetic as syn  # noqa: E402
 from cpz_b200.desc import (FLAG_IMPLICIT_DIFFUSION, FLAG_MPP, FLAG_SMOOTH_NN, FLAG_ZERO_WEIGHTS, RHS_INFER,  # noqa: E402
                            RHS_TRAIN, ClosureDesc, ClosureUvtDesc, NetDesc, RHS_EVALS)
 from oracle import nde  # noqa: E402
-from util import oracle_loss_grad, oracle_rhs, oracle_solve, rel_inf, t32, t64  # noqa: E402
+from util import (SPREAD_K, assert_block_errors, assert_blocks, field_blocks, oracle_loss_grad, oracle_rhs, oracle_solve,  # noqa: E402
+                  rel_inf, t32, t64, theta_blocks)
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -147,8 +148,9 @@ def drift_targets(d, x0):
     return mbs.bench_targets(d, x0)
 
 
-def assert_trajectories(got, ref, ref32, label):
-    """Worst column within max(1e-4, 3 x the FP32 oracle's worst column); Frobenius-norm error of the batch within 1e-4."""
+def assert_trajectories(d, got, ref, ref32, label):
+    """Worst column within max(1e-4, 3 x the FP32 oracle's worst column); Frobenius-norm error of the batch within 1e-4;
+    each field on its own within max(1e-4, 3 x the FP32 oracle's error on that field)."""
     n, sc = ref.shape[0], np.abs(ref).max()
     e = np.abs(got.astype(np.float64) - ref).reshape(n, -1).max(1) / sc
     f = np.abs(ref32.astype(np.float64) - ref).reshape(n, -1).max(1) / sc
@@ -159,6 +161,7 @@ def assert_trajectories(got, ref, ref32, label):
     assert np.isfinite(got).all()
     assert e.max() <= max(TOL, 3 * f.max()), (e.max(), f.max())
     assert e_fro <= TOL, e_fro
+    assert_blocks(label, got, ref, ref32, field_blocks(d), TOL, k=3.0)
 
 
 # ---- 1. tensor-core adjoint: reverse launches and record segments (FP64 golden) -----------------------------------------
@@ -171,7 +174,8 @@ def adj_case():
             d, th, x0, bcs, tgt = mbs.case_inputs(name)
             G = mbs.load(name)
             cache[name] = dict(d=d, th=th, x0=x0, bcs=bcs, tgt=tgt, tot=float(G["loss"][6]), g=G["grad"],
-                               floor_g=float(G["floor_grad"]), floor_l=float(G["floor_loss"]))
+                               floor_g=float(G["floor_grad"]), floor_l=float(G["floor_loss"]),
+                               floor_blocks=G["floor_grad_blocks"])
         return cache[name]
     return get
 
@@ -188,6 +192,11 @@ def _adj_assert(c, loss, grad, what):
     assert np.isfinite(grad).all()
     assert e_l <= max(TOL, c["floor_l"]), (what, e_l, c["floor_l"])
     assert e_g <= max(TOL, c["floor_g"]), (what, e_g, c["floor_g"])
+    # per (net, layer, W/b) block against the golden's per-block spread floors (util.assert_blocks: SPREAD_K x the largest
+    # FP32-oracle error at x0 and at ulp-nudged x0)
+    rows = [(name, np.linalg.norm(grad[sl] - c["g"][sl]) / np.linalg.norm(c["g"][sl]), SPREAD_K * floor, np.linalg.norm(c["g"][sl]))
+            for (name, sl), floor in zip(theta_blocks(c["d"]), c["floor_blocks"])]
+    assert_block_errors(what, rows, TOL)
 
 
 def test_adjoint_tc_several_reverse_launches_two_groups_per_cta(ctx, adj_case):
@@ -546,7 +555,7 @@ def test_tc_forward_tile_width_boundary(ctx, boundary_columns):
     out = {}
     for label, n in sizes.items():
         got = m.solve(c["x0"][:n], c["bcs"][:n])
-        assert_trajectories(got, c["ref"][:n], c["ref32"][:n], f"tcgen05 solve {label}: {cdiv(n, 28 if tc_forward_seven(n, sms) else 32)} tiles")
+        assert_trajectories(c["d"], got, c["ref"][:n], c["ref32"][:n], f"tcgen05 solve {label}: {cdiv(n, 28 if tc_forward_seven(n, sms) else 32)} tiles")
         out[n] = got
     m.close()
     # a column's arithmetic does not depend on the tile width it ran in
@@ -565,7 +574,7 @@ def test_tc_forward_implicit_diffusion_bench_config(ctx):
     assert "forward kernel: tcgen05" in m.describe()
     got = m.solve(x0, bcs)
     m.close()
-    assert_trajectories(got, oracle_solve(d, th, x0, bcs), oracle_solve(d, th, x0, bcs, dtype=torch.float32),
+    assert_trajectories(d, got, oracle_solve(d, th, x0, bcs), oracle_solve(d, th, x0, bcs, dtype=torch.float32),
                    "tcgen05 implicit-diffusion solve, 4096 columns")
 
 
@@ -584,6 +593,6 @@ def test_nnfree_default_four_columns_per_warp(ctx):
         got2 = m.solve(x0, bcs)
     m.close()
     ref, ref32 = oracle_solve(d, th, x0, bcs), oracle_solve(d, th, x0, bcs, dtype=torch.float32)
-    assert_trajectories(got, ref, ref32, f"nn-free {ncol} columns, 4 columns per warp")
+    assert_trajectories(d, got, ref, ref32, f"nn-free {ncol} columns, 4 columns per warp")
     # a column's arithmetic does not depend on how many columns its warp carries
     np.testing.assert_array_equal(got, got2)

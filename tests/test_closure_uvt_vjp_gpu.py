@@ -9,7 +9,7 @@ from cpz_b200 import engine, synthetic as syn, wind_mixing as wm
 from cpz_b200.desc import ClosureUvtDesc, FLAG_MPP, FLAG_SMOOTH_RI, RHS_INFER, RHS_TRAIN
 from oracle import nde
 from test_closure_uvt_vjp_oracle_cpu import mpp_of, oracle_closure_uvt, oracle_closure_uvt_vjp
-from util import rel_inf, t64
+from util import assert_blocks, mpp_blocks, mpp_scale, rel_inf, t64, theta_blocks
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -50,6 +50,9 @@ def _check(ctx, d, th, cd, u, v, T, fb, ob, label="", m=None):
         msg.append(f"{name} {err:.2e} (fp32-oracle {floor:.2e})")
         assert err <= max(TOL, floor), (name, err, floor)
     print("  ".join(msg))
+    assert_blocks("theta_bar", tb, ref[1], ref32[1], theta_blocks(d), TOL, norm="l2")
+    p = mpp_scale(d)
+    assert_blocks("mpp_bar", pb * p, ref[2] * p, ref32[2] * p, mpp_blocks(), TOL)
     return xb, tb, pb
 
 

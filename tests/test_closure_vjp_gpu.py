@@ -13,7 +13,7 @@ from cpz_b200 import engine, free_convection as fc, synthetic as syn
 from cpz_b200.desc import ClosureDesc, NetDesc, RHS_INFER
 from oracle import nde
 from test_closure_vjp_oracle_cpu import gyre_inputs, oracle_closure_vjp
-from util import rel_inf, t64
+from util import assert_blocks, rel_inf, t64, theta_blocks
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -85,6 +85,7 @@ def _check(ctx, d, th, cd, T, y, which, label="", m=None):
         msg.append(f"{name} {err:.2e} (fp32-oracle {floor:.2e})")
         assert err <= max(TOL, floor), (name, err, floor)
     print("  ".join(msg))
+    assert_blocks("theta_bar", tb, ref[1], ref32[1], theta_blocks(d), TOL, norm="l2")
     return fb, ob, Tb, tb
 
 

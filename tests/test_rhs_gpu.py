@@ -7,7 +7,7 @@ import torch
 from cpz_b200 import engine, synthetic as syn
 from cpz_b200.desc import (FLAG_CA, FLAG_CA_LITERAL_U, FLAG_DIURNAL, FLAG_DIURNAL_UNSHIFTED, FLAG_MPP, FLAG_SMOOTH_NN,
                            FLAG_SMOOTH_RI, FLAG_ZERO_WEIGHTS, RHS_INFER, RHS_TRAIN)
-from util import oracle_rhs, rel_inf
+from util import assert_blocks, field_blocks, oracle_rhs, rel_inf
 
 pytestmark = pytest.mark.gpu
 TOL_RHS = 1e-5
@@ -39,6 +39,7 @@ def _check(ctx, d, theta, ncol, t=0.37, use_q=False, seed=1000):
     print(f"rhs variant={d.variant} flags={d.flags} ncol={ncol}: cuda {err:.2e}  fp32-oracle {floor:.2e}")
     assert np.isfinite(got).all()
     assert err <= TOL_RHS, (err, floor)
+    assert_blocks("rhs", got, ref, ref32, field_blocks(d), TOL_RHS)
 
 
 @pytest.mark.parametrize("variant,flags", UVT_CASES)

@@ -12,7 +12,7 @@ from oracle import nde
 from test_jvp_oracle_cpu import oracle_rhs_jvp, p_of, tangents_of
 from test_rhs_gpu import UVT_CASES
 from test_rhs_vjp_gpu import ybar_of
-from util import rel_inf
+from util import assert_blocks, field_blocks, rel_inf
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-5
@@ -44,6 +44,7 @@ def _check(ctx, d, theta, ncol, t=0.37, use_q=False, seed=1000, label=""):
         err, floor = rel_inf(fd, r), rel_inf(r32, r)
         msg.append(f"{name} {err:.2e} (fp32-oracle {floor:.2e})")
         assert err <= max(TOL, floor), (name, err, floor)
+        assert_blocks(f"{name} tangent", fd, r, r32, field_blocks(d), TOL)
     m.close()
     print("  ".join(msg))
 

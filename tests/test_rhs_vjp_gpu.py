@@ -10,7 +10,8 @@ from cpz_b200.desc import (FLAG_CA, FLAG_DIURNAL, FLAG_IMPLICIT_DIFFUSION as IMP
                            FLAG_ZERO_WEIGHTS, RHS_INFER, RHS_TRAIN)
 from oracle import nde
 from test_rhs_gpu import UVT_CASES
-from util import oracle_loss_grad, oracle_solve, rel_inf
+from util import (assert_blocks, field_blocks, fp32_spread, mpp_blocks, mpp_scale, oracle_loss_grad, oracle_solve, rel_inf,
+                  theta_blocks, ulp_nudge)
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -62,6 +63,13 @@ def _check(ctx, d, theta, ncol, t=0.37, use_q=False, seed=1000, want_mpp=None, l
         msg.append(f"{name} {err:.2e} (fp32-oracle {floor:.2e})")
         assert err <= max(TOL, floor), (name, err, floor)
     print("  ".join(msg))
+    spread = fp32_spread(lambda s: oracle_rhs_vjp(d, theta, ulp_nudge(x, s), bcs, yb, t, Q, dtype=torch.float32, want_mpp=want_mpp))
+    assert_blocks("x_bar", xb, ref[0], ref32[0], field_blocks(d), TOL, spread=lambda: [r[0] for r in spread()])
+    if tb is not None:
+        assert_blocks("theta_bar", tb, ref[1], ref32[1], theta_blocks(d), TOL, norm="l2", spread=lambda: [r[1] for r in spread()])
+    if pb is not None:
+        p = mpp_scale(d)
+        assert_blocks("mpp_bar", pb * p, ref[2] * p, ref32[2] * p, mpp_blocks(), TOL, spread=lambda: [r[2] * p for r in spread()])
     return xb, tb, pb
 
 

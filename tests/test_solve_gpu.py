@@ -5,7 +5,7 @@ import torch
 
 from cpz_b200 import engine, synthetic as syn
 from cpz_b200.desc import FLAG_CA, FLAG_DIURNAL, FLAG_MPP, FLAG_ZERO_WEIGHTS, RHS_INFER, RHS_TRAIN
-from util import oracle_solve, rel_inf
+from util import assert_blocks, field_blocks, oracle_solve, rel_inf
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -25,6 +25,7 @@ def _check(ctx, d, theta, ncol, use_q=False):
     print(f"solve {d.integrator} steps={d.n_steps}x{d.n_substeps} ncol={ncol}: cuda {err:.2e} (final {err_final:.2e}) fp32-oracle {floor:.2e}")
     assert np.isfinite(got).all()
     assert err <= TOL, (err, floor)
+    assert_blocks("solve", got, ref, ref32, field_blocks(d), TOL)
     return got
 
 

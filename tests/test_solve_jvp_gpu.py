@@ -19,6 +19,7 @@ from oracle import nde
 from test_batch_schedules_gpu import _env
 from test_jvp_oracle_cpu import oracle_solve_jvp, p_of, tangents_of
 from test_solve_vjp_gpu import CASES, expected_path, rel_l2
+from util import assert_blocks, field_blocks
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -75,6 +76,7 @@ def test_solve_jvp_matches_the_oracle_and_each_adjoint_path(ctx, case):
     print(f"solve_jvp {case} ({path}) ncol={ncol}: traj_dot {err:.2e} (fp32-oracle {floor:.2e}); traj vs cpz_solve {e_p:.2e} "
           f"(fp32-oracle {f_p:.2e}); duality {e_dual:.2e} ({lhs:.6e} vs {rhs:.6e})")
     assert err <= max(TOL, 3.0 * floor), (err, floor)
+    assert_blocks("traj_dot", traj_dot, r, r32, field_blocks(d), TOL, k=3.0)
     assert e_p <= max(TOL, 3.0 * f_p), (e_p, f_p)
     assert e_dual <= max(DUAL_TOL, floor), (e_dual, floor)
 

@@ -10,7 +10,7 @@ import torch
 
 from cpz_b200 import engine, synthetic as syn
 from cpz_b200.desc import FLAG_CA, FLAG_DIURNAL, FLAG_MPP, FLAG_ZERO_WEIGHTS, RHS_INFER, RHS_TRAIN, NetDesc
-from util import oracle_rhs, oracle_solve, rel_inf
+from util import assert_blocks, field_blocks, oracle_rhs, oracle_solve, rel_inf
 
 pytestmark = pytest.mark.gpu
 
@@ -60,6 +60,7 @@ def test_tc_rhs_parity_net_shapes(ctx, h1, h2, act, variant):
     print(f"rhs h1={h1} h2={h2} {act} variant={variant}: tcgen05 {e_tc:.2e}  simt {e_simt:.2e}  tc-vs-simt {rel_inf(got, simt):.2e}")
     assert np.isfinite(got).all()
     assert e_tc <= 1e-5, (e_tc, e_simt)
+    assert_blocks("tcgen05 rhs", got, ref, oracle_rhs(d, th, x, bcs, 0.37, dtype=torch.float32), field_blocks(d), 1e-5)
 
 
 @pytest.mark.parametrize("flags,variant", [(FLAG_MPP | FLAG_ZERO_WEIGHTS, RHS_TRAIN), (FLAG_MPP, RHS_TRAIN), (FLAG_CA, RHS_TRAIN),
@@ -76,6 +77,7 @@ def test_tc_rhs_flags(ctx, flags, variant):
     m.close()
     ref = oracle_rhs(d, th, x, bcs, 0.21, Q)
     assert rel_inf(got, ref) <= 1e-5, rel_inf(got, ref)
+    assert_blocks("tcgen05 rhs", got, ref, oracle_rhs(d, th, x, bcs, 0.21, Q, dtype=torch.float32), field_blocks(d), 1e-5)
 
 
 @pytest.mark.parametrize("ncol", [1, 7, 16, 17, 32, 33, 100, 4096 + 5])
@@ -88,6 +90,7 @@ def test_tc_rhs_ragged_column_counts(ctx, ncol):
     m.close()
     ref = oracle_rhs(d, th, x, bcs, 0.0)
     assert got.shape == ref.shape and rel_inf(got, ref) <= 1e-5
+    assert_blocks("tcgen05 rhs", got, ref, oracle_rhs(d, th, x, bcs, 0.0, dtype=torch.float32), field_blocks(d), 1e-5)
 
 
 @pytest.mark.parametrize("integrator", ["euler", "rk4", "tsit5"])
@@ -106,6 +109,7 @@ def test_tc_solve_parity_and_agreement_with_simt(ctx, integrator):
     print(f"solve {integrator}: tcgen05 {e_tc:.2e}  simt {e_simt:.2e}  fp32-oracle {floor:.2e}")
     np.testing.assert_array_equal(got[:, 0], x0)
     assert e_tc <= 1e-4, (e_tc, e_simt, floor)
+    assert_blocks("tcgen05 solve", got, ref, ref32, field_blocks(d), 1e-4)
 
 
 def test_tc_solve_sharding_invariant_bitwise(ctx):
